@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- agent-steps/s of the mrs-gym step path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c5|c2|c3|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c5|c2|c3|c4] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Workload (default c5 = BASELINE.json configs[4], the config the metric is quoted on; it fits one
@@ -20,6 +20,11 @@ re-read from wherever the previous step left it (that is the real access pattern
 e2e: the same steps through mrs_step_host (C ABI, pinned HOST buffers): H2D actions, step, D2H of the
 newest X and A slices, stream sync -- every step.
 
+--dump-outputs DIR: after the timed region, what its last step handed the caller -- the newest X and A slices
+and the swarm state -- is written as DIR/<name>.npy (float32; rank 0's shard).  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.  The benchmark writes nothing else: the
+tree it runs from may be read-only.
+
 --impl reference: the CPU arm.  The reference is pure Python over PyBullet (not installable here,
 no network), so the CPU implementation that can run is the oracle port (oracle/spec.py, numpy,
 float64 Bullet restatement) on all host cores, one process per core, on a bounded sample of the
@@ -35,6 +40,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True      # no __pycache__ in the tree the benchmark runs from
 _REPO = os.path.dirname(os.path.abspath(__file__))
 for _p in (_REPO, os.path.join(_REPO, 'mrs-gym_b200'), os.path.join(_REPO, 'tests')):
     if _p not in sys.path:
@@ -261,6 +267,35 @@ def physical_gpu_index(local):
     return local
 
 
+# ------------------------------------------------------------------------------ --dump-outputs
+DUMP_BYTES = 64 * 10 ** 6     # at most this much in all (C5: 56.6 MB, written whole)
+
+
+def last_step_outputs(sw):
+    """What the timed path hands its caller after its last step, copied to the host: the newest slice of the
+    observation window X [E,N,6], of the adjacency window A [E,N,N] (absent with RETURN_A off) and the state
+    [E,N,13] (pos, quat xyzw, vel, angvel)."""
+    out = {'X': sw.X_window()[0], 'state': sw.state.t().reshape(sw.E, sw.N, -1)}
+    if sw.A_tape is not None:
+        out['A'] = sw.A_window()[0]
+    return {k: v.cpu().numpy() for k, v in out.items()}
+
+
+def dump_outputs(dirname, arrays, budget=DUMP_BYTES):
+    """DIR/<name>.npy for every array.  Larger than `budget` together: every array keeps the same fraction of its
+    rows (flattened to [rows, last axis]), picked with a fixed seed, so runs with the same arguments keep the same
+    rows."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in sorted(arrays.items()):
+        if total > budget:
+            rows = a.reshape(-1, a.shape[-1])
+            pick = np.random.default_rng(0).choice(len(rows), max(1, len(rows) * budget // total), replace=False)
+            a = rows[np.sort(pick)]
+        np.save(os.path.join(dirname, name + '.npy'), a)
+
+
 # ------------------------------------------------------------------------------ GPU arm
 def run_gpu(args):
     import numpy as np
@@ -360,6 +395,7 @@ def run_gpu(args):
         barrier()
         ms = e0.elapsed_time(e1)
         timed_stats = sw.read_stats()
+        outputs = last_step_outputs(sw) if args.dump_outputs else None
         # keep the same load running long enough for NVML to see the clocks under load
         t_end = time.time() + args.clock_seconds
         while time.time() < t_end:
@@ -491,6 +527,8 @@ def run_gpu(args):
         torch.distributed.destroy_process_group()
     if rank != 0:
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     peaks_path = os.path.join(_REPO, 'MEASURED_PEAKS.json')
     if os.path.isfile(peaks_path):
         peak, peak_src = float(json.load(open(peaks_path))['hbm_gbs']), 'measured (MEASURED_PEAKS.json hbm_gbs)'
@@ -627,7 +665,13 @@ def main():
     ap.add_argument('--clock-seconds', type=float, default=1.0)
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--envs', type=int, default=0, help='override envs per GPU (size sweeps; not the BASELINE config)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default='',
+                    help='write what the last timed step computed as DIR/<name>.npy (at most 64 MB)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs records the GPU path (--impl b200)')
     _quiet_stdout()
     if args.impl == 'reference':
         run_reference(args)

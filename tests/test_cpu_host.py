@@ -209,6 +209,28 @@ def test_reference_arm_prints_the_bench_contract():
     assert r1.returncode == 0 and r1.stdout.strip() == ''
 
 
+def test_bench_dump_outputs_within_the_budget(tmp_path):
+    """bench.py --dump-outputs: arrays are written whole when they fit the budget; otherwise every array keeps the
+    same fraction of its rows, the same rows on every run, and all of them together fit."""
+    import bench
+    rng = np.random.default_rng(1)
+    arrays = {'A': rng.random((2, 32, 64), dtype=np.float32), 'X': rng.random((2, 32, 6), dtype=np.float32)}
+    bench.dump_outputs(str(tmp_path / 'whole'), arrays)
+    for k, a in arrays.items():
+        np.testing.assert_array_equal(np.load(tmp_path / 'whole' / (k + '.npy')), a)
+    budget = 8000
+    for d in ('s1', 's2'):
+        bench.dump_outputs(str(tmp_path / d), arrays, budget=budget)
+    got = {k: np.load(tmp_path / 's1' / (k + '.npy')) for k in arrays}
+    assert 0 < sum(a.nbytes for a in got.values()) <= budget
+    total = sum(a.nbytes for a in arrays.values())
+    for k, a in got.items():
+        rows = arrays[k].reshape(-1, arrays[k].shape[-1])
+        assert a.dtype == np.float32 and a.shape == (len(rows) * budget // total, rows.shape[1])
+        assert all((rows == r).all(axis=1).any() for r in a)
+        np.testing.assert_array_equal(np.load(tmp_path / 's2' / (k + '.npy')), a)
+
+
 def test_plain_c_caller_links_and_runs(tmp_path):
     """examples/c_abi_smoke.c: a C99 program with no CUDA headers links against libmrs_b200.so and uses the
     configuration / validation entry points (the part of the ABI that needs no device)."""

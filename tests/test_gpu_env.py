@@ -446,3 +446,38 @@ def test_single_env_windows_stay_valid_without_a_copy_per_step():
     for (X, A), (Xr, Ar) in zip(held, want):
         assert torch.equal(X, Xr)
         assert A is None or torch.equal(A, Ar)
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs: two runs with the same arguments write the same arrays, and they are X, A and the state
+    after the warm-up replay and exactly --steps timed steps from the bench's start state."""
+    import json
+    import subprocess
+    import sys
+    import bench
+    import mrsgym_b200 as M
+    from conftest import _REPO
+    E, T = 256, 7
+    dumps = []
+    for i in range(2):
+        d = tmp_path / str(i)
+        r = subprocess.run([sys.executable, os.path.join(_REPO, 'bench.py'), '--envs', str(E), '--steps', str(T),
+                            '--warmup', '1', '--no-cpu', '--clock-seconds', '0', '--e2e-steps', '0', '--dump-outputs', str(d)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])['steps'] == T
+        dumps.append({k: np.load(d / (k + '.npy')) for k in ('X', 'A', 'state')})
+    a, b = dumps
+    for k in a:
+        assert a[k].dtype == np.float32 and np.array_equal(a[k], b[k]), k
+    # the same inputs through plain single-step launches: one warm-up replay of T steps, then the T timed steps
+    w = bench.WORKLOADS['c5']
+    st, act = bench.make_inputs(w, E, T, seed=1234 + 4)
+    sw = M.Swarm(E, w['N'], w['K'], w['mode'], M._abi.X_POS_VEL, w['R'])
+    H.upload_state(sw, st)
+    actions = torch.from_numpy(act).cuda()
+    for t in range(2 * T):
+        sw.step(actions[t % T])
+    np.testing.assert_array_equal(a['state'], sw.state.t().reshape(E, w['N'], 13).cpu().numpy())
+    np.testing.assert_array_equal(a['X'], sw.X_window()[0].cpu().numpy())
+    np.testing.assert_array_equal(a['A'], sw.A_window()[0].cpu().numpy())
