@@ -42,7 +42,7 @@
 extern "C" {
 #endif
 
-#define MRS_ABI_VERSION 3
+#define MRS_ABI_VERSION 4
 #define MRS_STATE_PLANES 13
 #define MRS_CTRL_PLANES 18
 #define MRS_STATS_SLOTS 8
@@ -85,6 +85,7 @@ typedef enum {
 #define MRS_STATUS_CONTACT_OVERFLOW 16u /* N > 32: an env had more agents / pairs in contact than the solver holds */
 #define MRS_STATUS_SYNC_TIMEOUT 8u /* a chained launch of mrs_rollout waited > 2 s for its predecessor's range    */
 #define MRS_STATUS_COMM_TIMEOUT 4u /* mrs_stats_allreduce / mrs_comm_barrier gave up waiting for a peer */
+#define MRS_STATUS_NEIGHBOR_OVERFLOW 32u /* mrs_neighbors: an agent had more neighbours than max_nbr (list truncated) */
 
 /* stats slots (unsigned long long, device; summed across GPUs per rollout) */
 #define MRS_STAT_AGENT_CONTACTS 0  /* sphere-sphere contact rows that pushed         */
@@ -93,6 +94,7 @@ typedef enum {
 #define MRS_STAT_NAN_ACTIONS 3
 #define MRS_STAT_CONTACT_CHUNKS 4   /* N <= 32: warp-chunk steps that took the contact path (solver) */
 #define MRS_STAT_SOLVER_SWEEPS 5    /* N <= 32: Gauss-Seidel sweeps summed over those chunk steps */
+#define MRS_STAT_NEIGHBOR_OVERFLOW 6 /* mrs_neighbors: rows whose list was truncated at max_nbr */
 
 /* cf2x.urdf properties (mrsgym/models/cf2x.urdf:5,11-12,42-78), the derived ones of
  * Quadcopter.calculate_parameters (Quadcopter.py:153-168) and the QuadControl gains
@@ -223,6 +225,21 @@ int mrs_observe(const MrsConfig* cfg, const MrsBuffers* bufs, int slot, int writ
 /* Adjacency of arbitrary float32 positions: pos device float[E][N][3] -> A float[E][N][N].
  * MRS.calc_A (MRS.py:117-124): bit-exact with torch CPU on identical positions. */
 int mrs_adjacency(const MrsConfig* cfg, const float* pos, float* A, void* stream);
+
+/* Neighbour lists of the COMM_RANGE graph of the current positions (bufs->state planes 0-2).
+ * For every agent i of every env:
+ *   cnt[e][i]              = number of j != i with A[e][i][j] == 1 (the exact predicate of
+ *                            mrs_adjacency / the step kernels, COMM_RANGE = inf included);
+ *   idx[e][i][0 .. min(cnt, max_nbr))
+ *                          = those j in ascending order; the remaining entries of the row are -1.
+ * idx: device int32 [E][N][max_nbr] (may be NULL when max_nbr == 0: degrees only);
+ * cnt: device int32 [E][N].  A degree above max_nbr keeps the first max_nbr neighbours, reports
+ * the true degree in cnt, sets MRS_STATUS_NEIGHBOR_OVERFLOW and adds the truncated rows to
+ * stats[MRS_STAT_NEIGHBOR_OVERFLOW] (max_nbr == 0 asks for the degrees alone and reports no
+ * overflow).  Deterministic, stream-ordered, capturable.  MRS_ERR_ARG for a negative max_nbr or a
+ * missing cnt, MRS_ERR_UNSUPPORTED when E * N * 32 does not fit in 32 bits.
+ * A graph learner's form of MRS.calc_A (MRS.py:117-124): 4 (max_nbr + 1) bytes per agent instead of 4 N. */
+int mrs_neighbors(const MrsConfig* cfg, const MrsBuffers* bufs, int max_nbr, int* idx, int* cnt, void* stream);
 
 /* Upload start states: device float[E][N][3] each (ori = euler 'xyz' roll,pitch,yaw), NULL
  * pointer = keep that component; env_mask device uint8[E] or NULL (= all envs).  PID state

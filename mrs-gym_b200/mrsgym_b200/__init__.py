@@ -9,7 +9,7 @@ registered there (reference: /root/reference/mrsgym/__init__.py:13-16).
 """
 from . import _abi
 from ._abi import MrsError
-from .core import Swarm, shard_range
+from .core import Swarm, Neighbors, shard_range
 from .env import MRS, Environment, AgentBatch
 from .spawn import DefaultSpawn, sample_start_pos
 from .rollout import rollout, reynolds_policy, to_trainer_history, save_dataset

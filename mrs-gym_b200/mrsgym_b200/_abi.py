@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('MRS_B200_LIB') or os.path.join(_HERE, 'libmrs_b200.so')   # override: A/B builds
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 STATE_PLANES = 13
 CTRL_PLANES = 18
 STATS_SLOTS = 8
@@ -33,9 +33,11 @@ STATUS_NONFINITE = 2
 STATUS_COMM_TIMEOUT = 4
 STATUS_SYNC_TIMEOUT = 8
 STATUS_CONTACT_OVERFLOW = 16
+STATUS_NEIGHBOR_OVERFLOW = 32
 COMM_MAX_WORLD = 16
 COMM_HANDLE_BYTES = 64
-STAT_NAMES = ('agent_contact_rows', 'ground_contacts', 'nonfinite', 'nan_actions', 'contact_chunks', 'solver_sweeps')
+STAT_NAMES = ('agent_contact_rows', 'ground_contacts', 'nonfinite', 'nan_actions', 'contact_chunks', 'solver_sweeps',
+              'neighbor_overflow')
 
 f = C.c_float
 
@@ -102,6 +104,7 @@ _SIGNATURES = {
                               C.c_void_p]),
     'mrs_observe': (C.c_int, [C.POINTER(MrsConfig), C.POINTER(MrsBuffers), C.c_int, C.c_int, C.c_int, C.c_void_p]),
     'mrs_adjacency': (C.c_int, [C.POINTER(MrsConfig), C.c_void_p, C.c_void_p, C.c_void_p]),
+    'mrs_neighbors': (C.c_int, [C.POINTER(MrsConfig), C.POINTER(MrsBuffers), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     'mrs_set_state': (C.c_int, [C.POINTER(MrsConfig), C.POINTER(MrsBuffers), C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.c_void_p, C.c_void_p]),
     'mrs_tape_fill': (C.c_int, [C.POINTER(MrsConfig), C.POINTER(MrsBuffers), C.c_int, C.c_int, C.c_int, C.c_int,

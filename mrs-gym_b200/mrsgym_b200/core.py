@@ -11,11 +11,15 @@ reference's newest-first K_HOPS+1 window (MRS.get_Xk / get_Ak, MRS.py:98-114) as
 view.  When a head reaches 0 the K newest slots are moved to the top of the tape.  X and A keep
 separate heads because the reference shifts its two deques independently (calc_Ak can be called
 without calc_Xk, examples/simulating_data/helper/DataGenerator.py:23).
+
+Neighbour mode (Swarm(..., neighbors=M)): the A tape is replaced by two int32 tapes, N_idx [L][E][N][M] and
+N_cnt [L][E][N] (mrs_neighbors), that follow the A head through every rule above.
 """
 from __future__ import annotations
 
 import ctypes as C
 import math
+from typing import NamedTuple
 
 import torch
 
@@ -39,6 +43,37 @@ def unpack_adjacency(bits, N: int):
     return ((b[..., j // 32] >> (j % 32)) & 1).to(torch.float32)
 
 
+class Neighbors(NamedTuple):
+    """The COMM_RANGE graph as neighbour lists (mrs_neighbors): idx int32 [..., N, M] holds the neighbours of every
+    agent in ascending order, padded with -1; count int32 [..., N] the true degree (count > M: the list was truncated
+    to its first M entries).  Windows of MRS are [E, K+1, N, M] / [E, K+1, N] (unbatched [K+1, N, M] / [K+1, N]),
+    newest first; a snapshot of Swarm.neighbors is [E, N, M] / [E, N]."""
+    idx: torch.Tensor
+    count: torch.Tensor
+
+    def to_dense(self):
+        """float32 {0,1} A [..., N, N] of the listed neighbours: the dense A of the same step when no row overflowed."""
+        idx = self.idx.long()
+        N = idx.shape[-2]
+        A = torch.zeros(*idx.shape[:-1], N + 1, dtype=torch.float32, device=idx.device)
+        A.scatter_(-1, torch.where(idx >= 0, idx, torch.full_like(idx, N)), 1.0)     # padding lands in column N
+        return A[..., :N].contiguous()
+
+    def edge_index(self, k=0):
+        """int64 [2, nnz] edge list of hop slice k over the node index e*N + i: edge_index[0] = i (the agent whose
+        list it is), edge_index[1] = j (its neighbour), in the row-major order of A.nonzero().  The graph is
+        symmetric, so this is also PyG's source -> target list.  idx [E, K+1, N, M] or [K+1, N, M] (one env);
+        k=None: no hop axis, [E, N, M] or [N, M] (a snapshot of Swarm.neighbors)."""
+        idx = self.idx
+        if k is not None:
+            idx = idx.select(-3, k)
+        N, M = idx.shape[-2], idx.shape[-1]
+        idx = idx.reshape(math.prod(idx.shape[:-1]), M).long()
+        rows = torch.arange(idx.shape[0], device=idx.device).unsqueeze(1).expand(-1, M)
+        keep = idx >= 0
+        return torch.stack([rows[keep], (rows - rows % N + idx)[keep]])
+
+
 def shard_range(E_total: int, rank: int, world: int):
     """Contiguous env block owned by `rank` (SURVEY.md §8e): [lo, hi)."""
     base, rem = divmod(E_total, world)
@@ -47,9 +82,19 @@ def shard_range(E_total: int, rank: int, world: int):
 
 
 class Swarm:
+    # neighbour mode (neighbors=M): lists per agent instead of the dense A tape (class defaults: dense mode)
+    nbr = None
+    N_idx = None
+    N_cnt = None
+
     def __init__(self, E: int, N: int, K: int = 0, action_type='set_target_vel', state_layout=_abi.X_POS_VEL,
                  comm_range=float('inf'), dt=0.01, gravity=9.81, agent_radius=0.3, device='cuda', contact_radius=None,
-                 tape_slots=None, want_A=True, custom_D=0, keep_rpm=False, ring=False, fresh_tapes=False):
+                 tape_slots=None, want_A=True, custom_D=0, keep_rpm=False, ring=False, fresh_tapes=False, neighbors=None):
+        """neighbors=M: the COMM_RANGE graph is kept as neighbour lists of at most M entries per agent (tapes N_idx
+        [L][E][N][M] / N_cnt [L][E][N], mrs_neighbors) and no dense A tape is allocated.  Every stepping call then
+        runs mrs_step without A followed by one mrs_neighbors launch per step, for every N: the one-launch
+        mrs_step_many and the chained hand-over of mrs_rollout (N <= 32) never store the intermediate positions
+        the lists are built from, so step_many / rollout / capture_rollout become per-step launches."""
         self.lib = _abi.lib()
         self.device = torch.device(device)
         if self.device.type != 'cuda':
@@ -62,6 +107,11 @@ class Swarm:
                                 'torch.cuda.set_device first (one process per GPU)' % (self.device, torch.cuda.current_device()))
         self.E, self.N, self.K = int(E), int(N), int(K)
         self.S = self.E * self.N
+        if neighbors is not None:
+            if int(neighbors) < 0:
+                raise ValueError('neighbors (list length M) must be >= 0')
+            self.nbr = int(neighbors)
+            want_A = False
         self.cfg = _abi.default_config()
         self.cfg.E, self.cfg.N, self.cfg.K = self.E, self.N, self.K
         self.set_action_type(action_type)
@@ -79,7 +129,7 @@ class Swarm:
             # a whole slice), so the move is amortised over L - K steps; deep tapes make it negligible.  Up to
             # 256 slots within a ~2 GB budget for X and A together (C5: 29 MB per slot -> 68 slots).
             D_ = _abi.STATE_DIMS[state_layout] if state_layout != _abi.X_NONE else int(custom_D)
-            slot_bytes = 4 * self.S * (max(D_, 0) + (self.N if want_A else 0))
+            slot_bytes = 4 * self.S * (max(D_, 0) + (self.N if want_A else 0) + (self.nbr + 1 if self.nbr is not None else 0))
             self.L = max(2 * self.K + 2, 16, min(256, int(2e9 // max(slot_bytes, 1))))
         if self.L < (self.K + 1 if ring else 2 * self.K + 2):
             raise ValueError('tape_slots must be >= 2*K_HOPS+2 (K_HOPS+1 in ring mode)')
@@ -93,6 +143,9 @@ class Swarm:
         self.rpm = torch.zeros(4, self.S, **z) if keep_rpm else None
         self.X_tape = torch.zeros(self.L, self.E, self.N, max(self.D, 1), **z) if self.D > 0 else None
         self.A_tape = torch.zeros(self.L, self.E, self.N, self.N, **z) if want_A else None
+        if self.nbr is not None:
+            self.N_idx = torch.full((self.L, self.E, self.N, self.nbr), -1, device=dev, dtype=torch.int32)
+            self.N_cnt = torch.zeros(self.L, self.E, self.N, device=dev, dtype=torch.int32)
         self.scratch = torch.zeros(self.lib.mrs_scratch_planes(self.E, self.N), self.S, **z) if self.N > 32 else None
         self.status = torch.zeros(1, device=dev, dtype=torch.int32)
         self.stats = torch.zeros(_abi.STATS_SLOTS, device=dev, dtype=torch.int64)
@@ -108,7 +161,7 @@ class Swarm:
         # the next slots come from a NEW tensor, so a window view handed out earlier is never overwritten and stays
         # valid for as long as somebody holds it (reference semantics: every step returns fresh tensors) without a
         # copy per step.  Only for small slots: one held view keeps its whole tape generation alive.
-        slot_bytes = 4 * self.S * (max(self.D, 0) + (self.N if want_A else 0))
+        slot_bytes = 4 * self.S * (max(self.D, 0) + (self.N if want_A else 0) + (self.nbr + 1 if self.nbr is not None else 0))
         self.fresh = bool(fresh_tapes) and not self.ring and slot_bytes * self.L <= (64 << 20)
         self.generation = 0        # bumped whenever a fresh tape replaces the current one
         self.a_empty = True        # no A slice pushed since the last full reset (MRS.py:186)
@@ -158,7 +211,16 @@ class Swarm:
         if self.ring:                # ring mode (graph rollouts): wrap around, nothing is moved
             return L
         tape = self.X_tape if which == 1 else self.A_tape
-        if tape is not None and self.fresh:
+        if which == 2 and self.N_idx is not None:     # neighbour tapes: torch copies of the K newest slots
+            if self.fresh:
+                new = (torch.empty_like(self.N_idx), torch.empty_like(self.N_cnt))
+                if K > 0:
+                    new[0][L - K:L], new[1][L - K:L] = self.N_idx[head:head + K], self.N_cnt[head:head + K]
+                self._swap_nbr(*new)
+            elif K > 0:
+                self.N_idx[L - K:L] = self.N_idx[head:head + K].clone()
+                self.N_cnt[L - K:L] = self.N_cnt[head:head + K].clone()
+        elif tape is not None and self.fresh:
             new = torch.empty_like(tape)
             if K > 0:
                 new[L - K:L] = tape[head:head + K]
@@ -187,11 +249,35 @@ class Swarm:
             self.bufs.A_tape = new.data_ptr()
         self.generation += 1
 
+    def _swap_nbr(self, new_idx, new_cnt):
+        self.N_idx, self.N_cnt = new_idx, new_cnt
+        self.generation += 1
+
+    def _has_A(self):
+        """An A history is kept: the dense A tape or the neighbour tapes."""
+        return self.A_tape is not None or self.N_idx is not None
+
+    def _push_neighbors(self, slot):
+        """mrs_neighbors of the current positions into neighbour-tape slot `slot`."""
+        S, M = self.S, self.nbr
+        idx = self.N_idx.data_ptr() + 4 * slot * S * M
+        rc = self.lib.mrs_neighbors(self._cfg_ref, self._bufs_ref, M, C.c_void_p(idx if M else 0),
+                                    C.c_void_p(self.N_cnt.data_ptr() + 4 * slot * S), self._stream())
+        if rc:
+            _abi.check(rc, 'mrs_neighbors')
+        self.launches += 1
+
     def renew_tapes(self):
         """Fresh-tape mode: continue on new tapes (the current windows move to their top), so that an in-place edit
         of the history -- a masked reset -- does not show through windows handed out earlier."""
         if not self.fresh:
             return
+        if self.N_idx is not None:
+            n = min(self.K + 1, self.L - self.ha)
+            new = (torch.empty_like(self.N_idx), torch.empty_like(self.N_cnt))
+            new[0][self.L - n:], new[1][self.L - n:] = self.N_idx[self.ha:self.ha + n], self.N_cnt[self.ha:self.ha + n]
+            self._swap_nbr(*new)
+            self.ha = self.L - n
         for which in (1, 2):
             tape = self.X_tape if which == 1 else self.A_tape
             if tape is None:
@@ -221,6 +307,8 @@ class Swarm:
                 self._swap_tape(1, torch.empty_like(self.X_tape))
             if self.A_tape is not None:
                 self._swap_tape(2, torch.empty_like(self.A_tape))
+            if self.N_idx is not None:
+                self._swap_nbr(torch.empty_like(self.N_idx), torch.empty_like(self.N_cnt))
         if self.X_tape is not None:
             if write_X and self.cfg.state_layout != _abi.X_NONE:
                 _abi.check(self.lib.mrs_observe(C.byref(self.cfg), C.byref(self.bufs), self.hx, 1, 0, st), 'mrs_observe')
@@ -234,6 +322,10 @@ class Swarm:
                        'mrs_tape_fill')
             self.launches += 1
             self.ha += 1          # empty deque: the first push lands on slot L-K-1
+        if self.N_idx is not None:    # empty window: no neighbours, cnt = 0
+            self.N_idx[self.ha:self.ha + K + 1].fill_(-1)
+            self.N_cnt[self.ha:self.ha + K + 1].zero_()
+            self.ha += 1
         self.a_empty = True
 
     def fill_X_history(self):
@@ -256,6 +348,21 @@ class Swarm:
 
     def A_window(self):
         return self._window(self.A_tape, self.ha)                 # [K+1, E, N, N]
+
+    def N_window(self):
+        """Neighbour mode: the newest-first K+1 window as Neighbors([K+1, E, N, M], [K+1, E, N])."""
+        return Neighbors(self._window(self.N_idx, self.ha), self._window(self.N_cnt, self.ha))
+
+    def neighbors(self, M):
+        """mrs_neighbors of the current positions, one-off (any mode): Neighbors([E, N, M], [E, N]).  A degree above
+        M sets STATUS_NEIGHBOR_OVERFLOW (read_status) and counts in read_stats()['neighbor_overflow']."""
+        M = int(M)
+        idx = torch.empty(self.E, self.N, M, dtype=torch.int32, device=self.device)
+        cnt = torch.empty(self.E, self.N, dtype=torch.int32, device=self.device)
+        _abi.check(self.lib.mrs_neighbors(self._cfg_ref, self._bufs_ref, M, _ptr(idx) if M else C.c_void_p(0), _ptr(cnt),
+                                          self._stream()), 'mrs_neighbors')
+        self.launches += 1
+        return Neighbors(idx, cnt)
 
     # ------------------------------------------------------------------ the step
     def _check_actions(self, actions, T=1, host=False):
@@ -281,6 +388,11 @@ class Swarm:
             raise ValueError('actions must start on a 16-byte boundary (got a view at offset %d of its storage); '
                              'pass actions.clone()' % actions.storage_offset())
 
+    def _dense_only(self, what):
+        if self.nbr is not None:
+            raise _abi.MrsError('%s copies dense A slices to the host; it has no neighbour-list form (build the swarm '
+                                'without neighbors=)' % what)
+
     def _step_launches(self, n=1, fused=False):
         """Kernels the library launches for n steps (bench: gpu_launches).  N <= 32: one fused kernel per step
         (per call when `fused`: mrs_step_many), plus one for a ragged last warp-chunk when N is 8, 16 or 32 and E
@@ -298,20 +410,25 @@ class Swarm:
         """One env.step for all envs.  actions: device float32 [E,N,A] contiguous, or None."""
         self._check_actions(actions)
         hx = self._make_room(1) - 1 if self.X_tape is not None else 0
-        ha = self._make_room(2) - 1 if self.A_tape is not None else 0
+        ha = self._make_room(2) - 1 if self._has_A() else 0
         rc = self._mrs_step(self._cfg_ref, self._bufs_ref, _ptr(actions), hx, ha, self._stream())
         if rc:
             _abi.check(rc, 'mrs_step')
         self.launches += self._launches_per_step
+        if self.nbr is not None:
+            self._push_neighbors(ha)
         if self.X_tape is not None:
             self.hx = hx
-        if self.A_tape is not None:
+        if self._has_A():
             self.ha = ha
             self.a_empty = False
 
     def step_many(self, actions, T: int):
-        """T steps with pre-computed actions [T,E,N,A]; chunks at tape wrap-arounds."""
+        """T steps with pre-computed actions [T,E,N,A]; chunks at tape wrap-arounds.  Neighbour mode: T steps of
+        step() (the lists need the positions of every step)."""
         self._check_actions(actions, T)
+        if self.nbr is not None:
+            return self.step_many_single(actions, T)
         done = 0
         while done < T:
             hx = self._make_room(1) if self.X_tape is not None else T
@@ -335,8 +452,11 @@ class Swarm:
 
     def rollout(self, actions, T: int):
         """mrs_rollout: T steps as T single-step launches issued by ONE C call; for N in {8, 16, 32} at scale the
-        launches are chained (range hand-over through `sync`, no grid-wide dependency).  Chunks at tape wrap-arounds."""
+        launches are chained (range hand-over through `sync`, no grid-wide dependency).  Chunks at tape wrap-arounds.
+        Neighbour mode: T steps of step() (mrs_step + mrs_neighbors each, never chained)."""
         self._check_actions(actions, T)
+        if self.nbr is not None:
+            return self.step_many_single(actions, T)
         done = 0
         while done < T:
             hx = self._make_room(1) if self.X_tape is not None else T
@@ -363,10 +483,14 @@ class Swarm:
         return GraphRollout(self, actions, T, stats_comm)
 
     def push_A(self):
-        """MRS.calc_Ak outside step: adjacency of the current positions becomes the newest slot."""
+        """MRS.calc_Ak outside step: adjacency (neighbour mode: the neighbour lists) of the current positions becomes
+        the newest slot."""
         ha = self._make_room(2) - 1
-        _abi.check(self.lib.mrs_observe(C.byref(self.cfg), C.byref(self.bufs), ha, 0, 1, self._stream()), 'mrs_observe')
-        self.launches += 1
+        if self.nbr is not None:
+            self._push_neighbors(ha)
+        else:
+            _abi.check(self.lib.mrs_observe(C.byref(self.cfg), C.byref(self.bufs), ha, 0, 1, self._stream()), 'mrs_observe')
+            self.launches += 1
         self.ha = ha
         self.a_empty = False
 
@@ -382,6 +506,7 @@ class Swarm:
         """mrs_step_host: pinned host actions in, newest X/A slice out, synchronous.  Abits_host (pinned int32
         [E,N,ceil(N/32)]) + dev_Abits (device staging of the same shape): the adjacency bit-packed for the wire."""
         self._check_actions(actions_host, host=True)
+        self._dense_only('step_host')
         hx = self._make_room(1) - 1 if self.X_tape is not None else 0
         ha = self._make_room(2) - 1 if self.A_tape is not None else 0
         _abi.check(self.lib.mrs_step_host(C.byref(self.cfg), C.byref(self.bufs), _ptr(actions_host), _ptr(dev_actions),
@@ -401,6 +526,7 @@ class Swarm:
         Chunks at tape wrap-arounds."""
         T = int(actions_host.shape[0])
         self._check_actions(actions_host, T, host=True)
+        self._dense_only('rollout_host')
         done = 0
         while done < T:
             hx = self._make_room(1) if self.X_tape is not None else T
@@ -618,7 +744,7 @@ class GraphRollout:
             # steps, so everything a later step can read is put back afterwards -- state, PID planes, counters
             # and the K+1 observation windows (the rest of the tapes is history nobody can reach any more)
             keep = [(t, t.clone()) for t in (sw.state, sw.ctrl, sw.status, sw.stats, sw.rpm) if t is not None]
-            for tape, which in ((sw.X_tape, 1), (sw.A_tape, 2)):
+            for tape, which in ((sw.X_tape, 1), (sw.A_tape, 2), (sw.N_idx, 2), (sw.N_cnt, 2)):
                 if tape is not None:
                     keep += [(tape[sl], tape[sl].clone()) for sl in sw.window_slots(which)]
             heads = (sw.hx, sw.ha, sw.a_empty, sw.launches)
@@ -636,7 +762,9 @@ class GraphRollout:
 
     def _body(self):
         sw = self.swarm
-        if sw.N > 32:
+        if sw.nbr is not None:
+            sw.step_many_single(self.actions, self.T)   # mrs_step + mrs_neighbors per step
+        elif sw.N > 32:
             sw.step_many(self.actions, self.T)       # wide path: per-step kernels anyway, adjacency overlapped
         else:
             sw.rollout(self.actions, self.T)             # single-step launches, chained where the shape allows

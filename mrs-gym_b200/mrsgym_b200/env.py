@@ -6,11 +6,17 @@ DT, GRAVITY, ...), same `step(actions, ACTION_TYPE=None) -> (X, reward, done, in
 info["A"], same callback order (update -> reward -> last_obs := X -> info -> done ->
 steps_since_reset += 1, MRS.py:260-274), same ring semantics (X padded with copies, A with
 zeros).  New kwargs: N_ENVS (batch of independent worlds; default 1 = reference shapes),
-DEVICE, TAPE_SLOTS, CHECK_NAN, COPY_OBS.
+DEVICE, TAPE_SLOTS, CHECK_NAN, COPY_OBS, A_FORMAT, MAX_NEIGHBORS.
 
 Shapes: N_ENVS == 1 -> X (K+1, N, D), A (K+1, N, N) exactly like the reference;
         N_ENVS  > 1 -> X [E, K+1, N, D], A [E, K+1, N, N] (zero-copy views of the device tapes
         unless COPY_OBS; a view stays valid for at least TAPE_SLOTS - 2*K_HOPS - 2 further steps).
+
+A_FORMAT='neighbors': get_Ak(), info['A'], the A= argument of the callbacks, calc_Ak() and refresh_A() return
+Neighbors windows instead of the dense A: idx [E, K+1, N, M] (neighbours in ascending order, -1 padded) and count
+[E, K+1, N] (unbatched [K+1, N, M] / [K+1, N]), newest first, M = MAX_NEIGHBORS (default min(N_AGENTS - 1, 64)).
+No dense A history is kept; calc_A() stays dense.  Neighbors.to_dense() gives the dense window back,
+Neighbors.edge_index(k) the edge list of hop k.
 """
 from __future__ import annotations
 
@@ -21,7 +27,7 @@ import numpy as np
 import torch
 
 from . import _abi
-from .core import Swarm
+from .core import Swarm, Neighbors
 from . import spawn as _spawn
 from .spaces import Box
 
@@ -187,6 +193,8 @@ class MRS:
         self.BATCHED = None          # None: batched shapes iff N_ENVS > 1
         self.SEED = 0                # seed of the on-device start-state sampler
         self.ENV_OFFSET = None       # global index of this process's first env; None: shard_range(rank) under torchrun
+        self.A_FORMAT = 'dense'      # 'neighbors': A windows as neighbour lists (Neighbors), no dense A history
+        self.MAX_NEIGHBORS = None    # list length M of A_FORMAT='neighbors'; None: min(N_AGENTS - 1, 64)
         self.set_constants(kwargs)
         if env != 'simple':
             raise NotImplementedError("only the 'simple' world (N x cf2x + ground plane, EnvCreator.py:7-13) is in scope")
@@ -252,10 +260,15 @@ class MRS:
             # probe the user's state_fn once on a throw-away one-env swarm to learn D
             probe = Swarm(1, self.N_AGENTS, 0, self.ACTION_TYPE, _abi.X_POS_VEL, device=self.DEVICE, want_A=False)
             custom_D = int(self._call_state_fn(probe).shape[-1])
+        if self.A_FORMAT not in ('dense', 'neighbors'):
+            raise ValueError("A_FORMAT must be 'dense' or 'neighbors', got %r" % (self.A_FORMAT,))
+        nbr = None
+        if self.A_FORMAT == 'neighbors':
+            nbr = min(self.N_AGENTS - 1, 64) if self.MAX_NEIGHBORS is None else int(self.MAX_NEIGHBORS)
         self.swarm = Swarm(self.N_ENVS, self.N_AGENTS, self.K_HOPS, self.ACTION_TYPE, layout, self.COMM_RANGE,
                            dt=self.sim.DT, gravity=self.sim.GRAVITY, agent_radius=self.AGENT_RADIUS,
                            device=self.DEVICE, tape_slots=self.TAPE_SLOTS, want_A=True, custom_D=custom_D,
-                           contact_radius=self.CONTACT_RADIUS, fresh_tapes=self._copy)
+                           contact_radius=self.CONTACT_RADIUS, fresh_tapes=self._copy, neighbors=nbr)
         self._clone = self._copy and not self.swarm.fresh      # fresh tapes: views stay valid, no copy per step
         self.STATE_SIZE = self.swarm.D
         self.ACTION_DIM = self.swarm.action_dim
@@ -344,7 +357,20 @@ class MRS:
         return self._window(1)
 
     def get_Ak(self):
+        if self.swarm.nbr is not None:
+            return self._nbr_window()
         return self._window(2)
+
+    def _nbr_window(self):
+        """Neighbors window in the reference's layout: [E, K+1, N, M] / [E, K+1, N] (unbatched [K+1, N, M] / [K+1, N])."""
+        idx, cnt = self.swarm.N_window()
+        if self._batched:
+            idx, cnt = idx.transpose(0, 1), cnt.transpose(0, 1)
+        else:
+            idx, cnt = idx[:, 0], cnt[:, 0]
+        if self._clone:
+            idx, cnt = idx.clone(), cnt.clone()
+        return Neighbors(idx, cnt)
 
     def calc_Xk(self):
         """MRS.calc_Xk (MRS.py:87-95): push X of the current state."""
@@ -368,6 +394,11 @@ class MRS:
         self._sync_cfg()
         sw = self.swarm
         m = torch.as_tensor(env_mask).to(sw.device).bool().reshape(sw.E)
+        if sw.nbr is not None:
+            new = sw.neighbors(sw.nbr)
+            sw.N_idx[sw.ha][m] = new.idx[m]
+            sw.N_cnt[sw.ha][m] = new.count[m]
+            return self.get_Ak()
         A0 = sw.adjacency(sw.get_pos())
         sw.A_tape[sw.ha][m] = A0[m]
         return self.get_Ak()
@@ -458,6 +489,10 @@ class MRS:
         if sw.A_tape is not None:
             for sl in sw.window_slots(2):
                 sw.A_tape[sl][m] = 0
+        if sw.N_idx is not None:
+            for sl in sw.window_slots(2):
+                sw.N_idx[sl][m] = -1
+                sw.N_cnt[sl][m] = 0
         Xk = self.get_Xk()
         self.last_obs = Xk
         return Xk
@@ -587,6 +622,9 @@ class MRS:
             raise Exception('The given action contains NaN')
         if v & _abi.STATUS_NONFINITE:
             raise FloatingPointError('simulation state left the finite range')
+        if v & _abi.STATUS_NEIGHBOR_OVERFLOW:
+            raise OverflowError('an agent had more neighbours within COMM_RANGE than MAX_NEIGHBORS = %d: its list was '
+                                'truncated (count holds the true degree); raise MAX_NEIGHBORS' % self.swarm.nbr)
 
     # ------------------------------------------------------------------ misc API parity
     def set_data(self, name, val):
