@@ -284,8 +284,9 @@ int mrs_spawn(const MrsConfig* cfg, const MrsBuffers* bufs, const unsigned char*
               float yaw_hi, int max_rounds, unsigned int* failed_envs, void* stream);
 
 /* Analytic sensors on the primitives of the 'simple' world (ground box top at ground_z, agents as
- * AGENT_RADIUS spheres: the contact geometry of the step), for all agents of all envs at once.
- * mrs_proximity: per agent the gap to the nearest other agent (centre distance - 2*AGENT_RADIUS) and
+ * phys.contact_radius spheres: the contact geometry of the step's pair rows; phys.agent_radius is only
+ * the spawn separation), for all agents of all envs at once.
+ * mrs_proximity: per agent the gap to the nearest other agent (centre distance - 2*contact_radius) and
  * its index, the gap of the collision cylinder to the ground, and collision = any gap < threshold
  * (the reference uses 0.04).  Any output pointer may be NULL.  Device arrays of E*N elements.
  * Replaces Object.collision / get_dist / get_contact_points distances (Object.py:98-140).

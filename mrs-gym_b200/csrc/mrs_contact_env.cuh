@@ -21,12 +21,15 @@ namespace mrs {
 // Limits: blockDim flagged agents and 4 * blockDim pairs per env (blockDim = N rounded up to a warp, <= 1024);
 // beyond that the surplus is left unsolved and MRS_STATUS_CONTACT_OVERFLOW is raised.
 constexpr int kIncident = 16;
-__host__ __device__ inline size_t contact_env_smem(int threads) {
-    return (size_t)threads * (4 + 12 + 12 + 4 + 2 * kIncident) + (size_t)(4 * threads) * (4 + 4 + 12) + 128 * 4;
+// words of the bit mask of occupied tournament rounds: rounds 0 .. N + (N & 1) - 2
+__host__ __device__ inline int contact_env_round_words(int N) { return (N + (N & 1) - 1 + 31) / 32; }
+__host__ __device__ inline size_t contact_env_smem(int threads, int N) {
+    return (size_t)threads * (4 + 12 + 12 + 4 + 2 * kIncident) + (size_t)(4 * threads) * (4 + 4 + 12) +
+           (size_t)contact_env_round_words(N) * 4;
 }
 
 // The CTA-wide body: every thread of the CTA calls it (CTA barriers inside) with the env's index; `smem_raw` is
-// contact_env_smem(blockDim.x) bytes of shared memory.  Reads v*, the pre-step positions and the flags from the
+// contact_env_smem(blockDim.x, c.N) bytes of shared memory.  Reads v*, the pre-step positions and the flags from the
 // scratch planes 0-6 and w* from the state planes 10-12, writes the solved v and w back there.
 static __device__ __noinline__ void contact_env_body(const MrsConfig& c, const Derived& d, const MrsBuffers& b, unsigned env,
                                               unsigned char* smem_raw) {
@@ -39,16 +42,16 @@ static __device__ __noinline__ void contact_env_body(const MrsConfig& c, const D
     unsigned* pr_ij = reinterpret_cast<unsigned*>(sv + 3 * cap);    // [pcap] lo | hi << 16 (local indices)
     int* pr_round = reinterpret_cast<int*>(pr_ij + pcap);           // [pcap] tournament round, later the level
     float* pr_lam = reinterpret_cast<float*>(pr_round + pcap);      // [pcap][3]
-    unsigned* rmask = reinterpret_cast<unsigned*>(pr_lam + 3 * pcap);   // [128] rounds that hold a pair
-    int* deg = reinterpret_cast<int*>(rmask + 128);                 // [cap] pairs of a flagged agent
+    const int N = c.N, tid = threadIdx.x, words = contact_env_round_words(N);
+    unsigned* rmask = reinterpret_cast<unsigned*>(pr_lam + 3 * pcap);   // [words] rounds that hold a pair
+    int* deg = reinterpret_cast<int*>(rmask + words);               // [cap] pairs of a flagged agent
     unsigned short* inc = reinterpret_cast<unsigned short*>(deg + cap);     // [cap][kIncident] their indices
-    const int N = c.N, tid = threadIdx.x;
     const size_t S = (size_t)c.E * N, env0 = (size_t)env * N;
     const MrsPhysicsParams& ph = c.phys;
     const ContactParams cp = make_contact_params(ph, d);
     const float* __restrict__ sc = b.scratch;
     if (tid == 0) { n_flag = 0; n_pair = 0; deg_over = 0; max_level = 0; }
-    if (tid < 128) rmask[tid] = 0u;
+    for (int w = tid; w < words; w += blockDim.x) rmask[w] = 0u;
     deg[tid] = 0;
     __syncthreads();
     for (int i = tid; i < N; i += blockDim.x)
@@ -140,7 +143,6 @@ static __device__ __noinline__ void contact_env_body(const MrsConfig& c, const D
         if (top) atomicMax(&max_level, top);
         __syncthreads();
     }
-    const int words = (N + (N & 1) - 1 + 31) / 32;
     const int levels = max_level;
     auto solve_pair = [&](int k) -> float {
         const int lo = pr_ij[k] & 0xffffu, hi = pr_ij[k] >> 16;

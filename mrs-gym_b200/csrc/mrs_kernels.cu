@@ -263,8 +263,8 @@ spawn_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const Spaw
 }
 
 // ------------------------------------------------------------------------------ sensors (row f4)
-// Analytic sensors of the 'simple' world (ground box top at ground_z, agents as AGENT_RADIUS
-// spheres -- the same contact geometry as the step).  One thread per agent (proximity) or per
+// Analytic sensors of the 'simple' world (ground box top at ground_z, agents as CONTACT_RADIUS
+// spheres -- the same contact geometry as the step; AGENT_RADIUS is only the spawn separation).  One thread per agent (proximity) or per
 // (agent, ray) (raycast); partners are walked from the L1/L2-resident position planes.
 // Object.collision / get_dist / get_contact_points / raycast (Object.py:100-174) on these primitives.
 __global__ void __launch_bounds__(128)
@@ -288,7 +288,7 @@ proximity_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, float 
         const float d2 = dx * dx + dy * dy + dz * dz;
         if (d2 < best) { best = d2; arg = j; }
     }
-    const float ga = sqrtf(best) - 2.f * c.phys.agent_radius;
+    const float ga = sqrtf(best) - 2.f * c.phys.contact_radius;
     // ground: same support extent of the collision cylinder as the contact row of the step
     const float qx = b.state[3 * (size_t)S + s], qy = b.state[4 * (size_t)S + s];
     const float R22 = 1.f - 2.f * (qx * qx + qy * qy);
@@ -342,7 +342,7 @@ raycast_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const fl
     const float* px = b.state + env0;
     const float* py = b.state + (size_t)S + env0;
     const float* pz = b.state + 2 * (size_t)S + env0;
-    const float rad2 = c.phys.agent_radius * c.phys.agent_radius;
+    const float rad2 = c.phys.contact_radius * c.phys.contact_radius;
     for (int j = 0; j < N; ++j) {
         if (j == ai) continue;
         const float cx = px[j] - sx, cy = py[j] - sy, cz = pz[j] - sz;
@@ -430,15 +430,15 @@ int launch_contact_env(const MrsConfig& c, const Derived& d, const MrsBuffers& b
     if (!c.phys.agent_contact || c.N < 2) return MRS_OK;
     int threads = (c.N + 31) / 32 * 32;
     if (threads > 1024) threads = 1024;
-    const size_t smem = contact_env_smem(threads);
-    static bool configured[64] = {};
+    const size_t smem = contact_env_smem(threads, c.N);
+    // the round mask grows with N: raise the kernel's dynamic shared-memory limit to the largest size asked for
+    static size_t configured[64] = {};
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return MRS_ERR_CUDA;
-    if (!configured[dev]) {
-        if (cudaFuncSetAttribute(contact_env_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)contact_env_smem(1024)) != cudaSuccess)
+    if (smem > configured[dev]) {
+        if (cudaFuncSetAttribute(contact_env_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
             return MRS_ERR_CUDA;
-        configured[dev] = true;
+        configured[dev] = smem;
     }
     return launch_pdl(pdl, contact_env_kernel, dim3((unsigned)c.E), (unsigned)threads, smem, st, c, d, b);
 }

@@ -1454,7 +1454,7 @@ static int launch_env_fused(const MrsConfig& c, const Derived& d, const MrsBuffe
     const size_t S = (size_t)c.E * c.N;
     constexpr int A = ModeTraits<MODE>::A;
     const unsigned threads = (unsigned)((c.N + 31) / 32 * 32);
-    const size_t smem = contact_env_smem((int)threads);
+    const size_t smem = contact_env_smem((int)threads, c.N);
     for (int t = 0; t < a.T; ++t) {
         const float* act_t = a.actions ? a.actions + (size_t)t * S * A : nullptr;
         float* A_slice = b.A_tape ? b.A_tape + (size_t)(a.slot_a - t) * S * c.N : nullptr;

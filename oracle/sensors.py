@@ -2,7 +2,8 @@
 
 Restates Object.collision / get_dist / raycast (/root/reference/mrsgym/Object.py:98-174) on the
 primitives the B200 step uses for contact: ground = top face (z = ground_z, |x|,|y| <= 15) of the
-30 x 30 x 1 box of plane.urdf:21-26, agents = AGENT_RADIUS spheres (north star's contact geometry),
+30 x 30 x 1 box of plane.urdf:21-26, agents = CONTACT_RADIUS spheres (the spheres the step's pair rows use;
+AGENT_RADIUS is only the spawn separation),
 the quad's own ground gap = collision-cylinder support extent as in bullet_model.ground_contact.
 PARITY UNPINNED against PyBullet: the reference answers these queries on Bullet's hull geometry
 (getClosestPoints / rayTestBatch), which cannot be run here; this is the specification the kernels
@@ -22,7 +23,7 @@ def proximity(pos, quat, P: bm.PhysicsParams, threshold=0.04):
     d = np.linalg.norm(pos[:, :, None, :] - pos[:, None, :, :], axis=-1)
     d[:, np.arange(N), np.arange(N)] = np.inf
     nearest = np.where(N > 1, d.argmin(axis=-1), -1)
-    gap_agent = d.min(axis=-1) - 2.0 * P.agent_radius
+    gap_agent = d.min(axis=-1) - 2.0 * P.contact_radius
     R22 = bm.quat_to_mat(np.asarray(quat, np.float64))[..., 2, 2]
     ext = P.col_radius * np.sqrt(np.maximum(1 - R22 * R22, 0)) + P.col_halfheight * np.abs(R22) + P.col_margin
     gap_ground = pos[..., 2] - ext - P.ground_z
@@ -59,9 +60,9 @@ def raycast(pos, quat, directions, offset, body, rng, P: bm.PhysicsParams):
                     c = pos[e, j] - s
                     tc = c @ dvec
                     d2 = c @ c - tc * tc
-                    if d2 > P.agent_radius ** 2:
+                    if d2 > P.contact_radius ** 2:
                         continue
-                    t = tc - np.sqrt(P.agent_radius ** 2 - d2)
+                    t = tc - np.sqrt(P.contact_radius ** 2 - d2)
                     if 0 <= t < best:
                         best, bid = t, j
                 if bid >= 0:
