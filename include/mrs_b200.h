@@ -271,12 +271,17 @@ int mrs_step_host(const MrsConfig* cfg, const MrsBuffers* bufs, const float* act
 int mrs_pack_adjacency(const MrsConfig* cfg, const float* A, unsigned int* bits, void* stream);
 
 /* On-device reset with the reference's DEFAULT start distribution for the envs selected by
- * env_mask (NULL = all): positions z ~ U[z_lo, z_hi], xy ~ N(0, xy_sigma) pulled onto the disc of
- * radius xy_radius, re-drawn until all agents of an env are >= 2*AGENT_RADIUS apart (at most
- * max_rounds rounds; envs that did not converge are counted in *failed_envs, device u32, may be
- * NULL); yaw ~ U[yaw_lo, yaw_hi], roll = pitch = 0; velocities zero.  Counter-based RNG: the result
- * depends on (seed, env_offset + env index) only -- env_offset is the global index of this shard's first env, so
- * the ranks of a sharded job draw different environments from one seed.  N <= 32.
+ * env_mask (NULL = all; only the 13 state planes of the selected envs are written), any N.
+ * Round 0: every agent draws xy ~ N(0, xy_sigma) pulled onto the disc of radius xy_radius and z ~ U[z_lo, z_hi];
+ * then agent i is flagged iff some j < i of its env is closer than 2*AGENT_RADIUS (squared distance < 4 r^2,
+ * this round's positions).  Every later round re-draws the flagged agents and tests again; an env stops when no
+ * agent is flagged.  An env still flagged after max_rounds rounds keeps its last positions and counts once in
+ * *failed_envs (device u32, added to, may be NULL).  yaw ~ U[yaw_lo, yaw_hi], roll = pitch = 0; velocities zero.
+ * Counter-based RNG (splitmix64 keyed by seed, global env index env_offset + e, agent and round): the result
+ * depends on (seed, env_offset + e, N, the spawn arguments, AGENT_RADIUS) only, not on E, env_mask or the launch
+ * shape -- env_offset is the global index of this shard's first env, so the ranks of a sharded job draw
+ * different environments from one seed.  N <= 32 and N > 32 use different key packings (a warp per env / a CTA
+ * per env), so their streams differ.  E*N must fit 32-bit slot indices (MRS_ERR_UNSUPPORTED otherwise).
  * Replaces MRS.generate_start_pos / generate_start_ori / default_spawn_dist + the set_state of
  * MRS.reset (MRS.py:69-78,127-161,174-184) without the host round trip. */
 int mrs_spawn(const MrsConfig* cfg, const MrsBuffers* bufs, const unsigned char* env_mask,

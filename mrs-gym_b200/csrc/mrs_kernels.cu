@@ -262,6 +262,115 @@ spawn_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const Spaw
     for (int p = 7; p < 13; ++p) st[p * (size_t)S + s] = 0.f;
 }
 
+// Wide form (N > 32): one CTA per env, the same draws and the same rejection rule, stated per agent: in round r
+// every agent flagged in round r - 1 (all of them in round 0) draws again, then agent i is flagged iff some j < i
+// lies closer than 2*AGENT_RADIUS in this round's positions.  The positions live in the env's state planes (L2),
+// the per-agent "drew this round" and "flagged" bits in ceil(N/32)-word masks in dynamic shared memory, so N is
+// bounded only by that (~900K agents).
+// After round 0 a pair of two agents that did not draw was tested in the previous round with the same positions
+// and found apart (else the higher one would have drawn), so only pairs with a mover are tested: for every mover a,
+// (a, k) for all k > a and, after round 0, for the non-movers k < a (mover pairs once).  A round costs
+// movers x N pair tests; the flags are those of the full rule.
+// The warp kernel's key packing aliases at agent >= 256 or round >= 4096, so this kernel packs (agent, round) into
+// one 64-bit word under a per-env hash; round 0xFFFFFFFF (never drawn: max_rounds is an int) is the yaw's domain.
+__device__ __forceinline__ unsigned long long spawn_wide_key(unsigned long long seed, unsigned long long env_hash,
+                                                             unsigned agent, unsigned round) {
+    return splitmix64(seed ^ splitmix64(env_hash ^ (((unsigned long long)agent << 32) | round)));
+}
+
+__global__ void __launch_bounds__(1024)
+spawn_wide_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const SpawnArgs sp,
+                  const unsigned char* __restrict__ mask, unsigned* __restrict__ failed) {
+    extern __shared__ unsigned spawn_bits[];
+    const unsigned e = blockIdx.x;
+    if (mask && !mask[e]) return;
+    const int N = c.N;
+    const int W = (N + 31) / 32;
+    unsigned* moved = spawn_bits;          // agents that draw in this round
+    unsigned* flag = spawn_bits + W;       // agents flagged by this round's test
+    const size_t S = (size_t)c.E * (size_t)N;
+    float* px = b.state + (size_t)e * N;
+    float* py = px + S;
+    float* pz = py + S;
+    const float lim2 = 4.f * c.phys.agent_radius * c.phys.agent_radius;
+    const unsigned long long env_hash = splitmix64(sp.env_offset + (unsigned long long)e);
+    for (int w = threadIdx.x; w < W; w += blockDim.x) moved[w] = (w == W - 1 && (N & 31)) ? (1u << (N & 31)) - 1u : kFull32;
+    __syncthreads();
+    int round = 0;
+    for (; round < sp.max_rounds; ++round) {
+        for (int i = threadIdx.x; i < N; i += blockDim.x) {
+            if (!((moved[i >> 5] >> (i & 31)) & 1u)) continue;
+            const unsigned long long key = spawn_wide_key(sp.seed, env_hash, (unsigned)i, (unsigned)round);
+            const float u1 = u01(key), u2 = u01(splitmix64(key)), u3 = u01(splitmix64(key ^ 0x5851F42D4C957F2Dull));
+            const float r = sp.xy_sigma * sqrtf(-2.f * logf(u1));          // Box-Muller
+            float sn, cs;
+            sincosf(6.28318530717958647692f * u2, &sn, &cs);
+            float x = r * cs, y = r * sn;
+            const float mag = fmaxf(sqrtf(x * x + y * y), sp.xy_radius);     // SphereTransform(within=True)
+            x = x / mag * sp.xy_radius; y = y / mag * sp.xy_radius;
+            px[i] = x; py[i] = y; pz[i] = sp.z_lo + (sp.z_hi - sp.z_lo) * u3;
+        }
+        for (int w = threadIdx.x; w < W; w += blockDim.x) flag[w] = 0u;
+        __syncthreads();                   // this round's positions and the cleared flags are visible to the CTA
+        for (int w = 0; w < W; ++w) {
+            for (unsigned bits = moved[w]; bits; bits &= bits - 1u) {
+                const int a = 32 * w + __ffs(bits) - 1;
+                const float xa = px[a], ya = py[a], za = pz[a];
+                for (int k = a + 1 + threadIdx.x; k < N; k += blockDim.x) {
+                    const float dx = xa - px[k], dy = ya - py[k], dz = za - pz[k];
+                    if (dx * dx + dy * dy + dz * dz < lim2) atomicOr(&flag[k >> 5], 1u << (k & 31));
+                }
+                if (round == 0) continue;
+                bool hit = false;
+                for (int k = threadIdx.x; k < a; k += blockDim.x) {
+                    if ((moved[k >> 5] >> (k & 31)) & 1u) continue;
+                    const float dx = xa - px[k], dy = ya - py[k], dz = za - pz[k];
+                    hit = hit || dx * dx + dy * dy + dz * dz < lim2;
+                }
+                if (hit) atomicOr(&flag[a >> 5], 1u << (a & 31));
+            }
+        }
+        __syncthreads();
+        int any = 0;
+        for (int w = threadIdx.x; w < W; w += blockDim.x) {
+            moved[w] = flag[w];
+            any |= flag[w] != 0u;
+        }
+        if (!__syncthreads_or(any)) break;
+    }
+    if (round >= sp.max_rounds && threadIdx.x == 0 && failed) atomicAdd(failed, 1u);
+    float* st = b.state + (size_t)e * N;
+    for (int i = threadIdx.x; i < N; i += blockDim.x) {
+        const unsigned long long ky = spawn_wide_key(sp.seed, env_hash, (unsigned)i, 0xFFFFFFFFu);
+        const float yaw = sp.yaw_lo + (sp.yaw_hi - sp.yaw_lo) * u01(ky);
+        float sy, cy;
+        sincosf(0.5f * yaw, &sy, &cy);
+        st[3 * S + i] = 0.f; st[4 * S + i] = 0.f; st[5 * S + i] = sy; st[6 * S + i] = cy;
+#pragma unroll
+        for (int p = 7; p < 13; ++p) st[p * S + i] = 0.f;
+    }
+}
+
+static int launch_spawn_wide(const MrsConfig& c, const MrsBuffers& b, const SpawnArgs& sp, const unsigned char* mask,
+                             unsigned* failed, cudaStream_t st) {
+    int threads = (c.N + 31) / 32 * 32;
+    if (threads > 1024) threads = 1024;
+    const size_t smem = 2 * (size_t)((c.N + 31) / 32) * sizeof(unsigned);
+    // the two bit masks grow with N: raise the kernel's dynamic shared-memory limit to the largest size asked for
+    static size_t configured[64] = {};
+    int dev = 0, optin = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return MRS_ERR_CUDA;
+    if (smem > configured[dev] && smem > 48 * 1024) {
+        if (cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess) return MRS_ERR_CUDA;
+        if (smem > (size_t)optin) return MRS_ERR_UNSUPPORTED;
+        if (cudaFuncSetAttribute(spawn_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return MRS_ERR_CUDA;
+        configured[dev] = smem;
+    }
+    spawn_wide_kernel<<<(unsigned)c.E, (unsigned)threads, smem, st>>>(c, b, sp, mask, failed);
+    return last_error();
+}
+
 // ------------------------------------------------------------------------------ sensors (row f4)
 // Analytic sensors of the 'simple' world (ground box top at ground_z, agents as CONTACT_RADIUS
 // spheres -- the same contact geometry as the step; AGENT_RADIUS is only the spawn separation).  One thread per agent (proximity) or per
@@ -946,11 +1055,13 @@ int mrs_spawn(const MrsConfig* cfg, const MrsBuffers* bufs, const unsigned char*
     int rc = check_cfg(cfg);
     if (rc) return rc;
     if (!bufs || !bufs->state) return MRS_ERR_ARG;
-    if (cfg->N > 32) return MRS_ERR_UNSUPPORTED;
     if (!(z_hi >= z_lo) || !(xy_radius > 0.f) || !(xy_sigma > 0.f) || max_rounds <= 0) return MRS_ERR_ARG;
+    if ((size_t)cfg->E * (size_t)cfg->N > 0xffffffffull) return MRS_ERR_UNSUPPORTED;     // u32 slot indices
     SpawnArgs sp;
     sp.seed = seed; sp.env_offset = env_offset; sp.z_lo = z_lo; sp.z_hi = z_hi; sp.xy_radius = xy_radius; sp.xy_sigma = xy_sigma;
     sp.yaw_lo = yaw_lo; sp.yaw_hi = yaw_hi; sp.max_rounds = max_rounds;
+    // a warp per env packs 4 envs into a CTA; past 32 agents an env takes a CTA of its own
+    if (cfg->N > 32) return launch_spawn_wide(*cfg, *bufs, sp, env_mask, failed_envs, (cudaStream_t)stream);
     spawn_kernel<<<(unsigned)((cfg->E + 3) / 4), 128, 0, (cudaStream_t)stream>>>(*cfg, *bufs, sp, env_mask, failed_envs);
     return last_error();
 }

@@ -566,10 +566,12 @@ class Swarm:
 
     def spawn(self, seed, env_mask=None, z=(1.0, 3.0), xy_radius=1.0, xy_sigma=1.0, yaw=(-math.pi / 2, math.pi / 2),
               max_rounds=256, env_offset=0):
-        """On-device reset with the reference's default start distribution (mrs_spawn).  env_offset: global index
-        of this shard's first env (the draws are keyed by seed and GLOBAL env index, so the ranks of a sharded job
-        sample different environments).  Returns the device counter of envs whose rejection sampling did not
-        converge (read it lazily)."""
+        """On-device reset with the reference's default start distribution (mrs_spawn), any N: a warp per env for
+        N <= 32, a CTA per env above.  Agents closer than 2*agent_radius to a lower-indexed agent of their env are
+        re-drawn, for at most max_rounds rounds.  env_offset: global index of this shard's first env (the draws are
+        keyed by seed and GLOBAL env index, so the ranks of a sharded job sample different environments; the result
+        does not depend on E or env_mask).  Returns the device counter of envs whose rejection sampling did not
+        converge within max_rounds (read it lazily); those envs keep their last draw."""
         if env_mask is not None:
             env_mask = torch.as_tensor(env_mask).to(self.device).to(torch.uint8).reshape(self.E).contiguous()
         failed = torch.zeros(1, device=self.device, dtype=torch.int32)

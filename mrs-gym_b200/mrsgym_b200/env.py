@@ -458,7 +458,7 @@ class MRS:
 
     def _device_spawn_ok(self):
         """The default START_POS / START_ORI (MRS.py:53-54) can be sampled on the device."""
-        if not isinstance(self.START_POS, _spawn.DefaultSpawn) or self.N_AGENTS > 32:
+        if not isinstance(self.START_POS, _spawn.DefaultSpawn):
             return False
         ori = torch.as_tensor(self.START_ORI, dtype=torch.float32)
         if ori.dim() != 2 or ori.shape[-1] != 6:
@@ -506,9 +506,15 @@ class MRS:
             ori6 = torch.as_tensor(self.START_ORI, dtype=torch.float32)[0]
             sp = self.START_POS
             self._spawn_count += 1
+            # N > 32 keeps the host sampler's failure contract (10000 rounds, then RuntimeError): one synchronising
+            # read of the counter per reset.  N <= 32 keeps its lazy counter and 256 rounds.
+            wide = self.N_AGENTS > 32
             self.spawn_failed = self.swarm.spawn(self.SEED * 1000003 + self._spawn_count, env_mask=env_mask,
                                                  z=(sp.z_low, sp.z_high), xy_radius=sp.xy_radius, xy_sigma=sp.xy_radius,
-                                                 yaw=(float(ori6[2]), float(ori6[5])), env_offset=self._env_offset())
+                                                 yaw=(float(ori6[2]), float(ori6[5])), env_offset=self._env_offset(),
+                                                 max_rounds=10000 if wide else 256)
+            if wide and int(self.spawn_failed.item()):
+                raise RuntimeError('start-position rejection sampling did not converge (N_AGENTS too dense for START_POS)')
             if vel is not None or angvel is not None:
                 self.swarm.set_state(vel=vel, angvel=angvel, env_mask=env_mask)
         else:
