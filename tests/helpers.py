@@ -89,6 +89,41 @@ def spec_state(env):
     return dict(pos=env.pos.copy(), quat=env.quat.copy(), vel=env.vel.copy(), angvel=env.angvel.copy())
 
 
+# One-step delta bar of the parity tests: |d_gpu - d_ref| <= REL * |d_ref| + floor, both deltas measured from the
+# common float32 start state; the floor is the float32 resolution of the stored quantity (pos: also one ulp of the
+# coordinate)
+REL = 1e-4
+FLOOR = dict(pos=5e-7, vel=5e-7, angvel=1e-5, quat=3e-7)
+
+
+def delta_ratio(s0, r1, g1):
+    """{quantity: largest |(g1 - s0) - (r1 - s0)| in multiples of the bar around the reference r1}"""
+    worst = {}
+    for k in ('pos', 'vel', 'angvel', 'quat'):
+        base = s0[k].astype(np.float64)
+        dg, dr = g1[k] - base, r1[k] - base
+        if k == 'quat':       # q and -q are the same rotation
+            flip = np.sum(g1[k] * r1[k], axis=-1, keepdims=True) < 0
+            dg = np.where(flip, -g1[k], g1[k]) - base
+        err = np.abs(dg - dr)
+        floor = FLOOR[k]
+        if k == 'pos':     # one float32 ulp of the stored coordinate (5e-7 m up to 8 m, 1e-6 m up to 16 m, ...)
+            floor = np.maximum(floor, np.spacing(np.abs(g1[k]).astype(np.float32)).astype(np.float64))
+        tol = REL * np.abs(dr) + floor
+        worst[k] = float(np.max(err / tol)) if err.size else 0.0
+        if not np.all(np.isfinite(err)):
+            worst[k] = float('inf')
+    return worst
+
+
+def check_delta(tag, s0, g1, r1):
+    """one-step deltas, GPU (g1) vs oracle (r1), both measured from the common start state s0"""
+    worst = delta_ratio(s0, r1, g1)
+    for k, w in worst.items():
+        assert w <= 1.0, '%s: %s delta off by %.3g x tolerance' % (tag, k, w)
+    return worst
+
+
 def quat_angle(q1, q2):
     """Rotation angle between unit quaternions (rad), sign-insensitive."""
     d = np.abs(np.sum(q1 * q2, axis=-1)) / (np.linalg.norm(q1, axis=-1) * np.linalg.norm(q2, axis=-1))

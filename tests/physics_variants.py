@@ -17,15 +17,10 @@ PHYS_FIELDS = {
     'solver_tol': 'solver_tol',
 }
 
-# MrsPhysicsParams fields no variant sets, and why
+# MrsPhysicsParams fields neither these variants nor the free-flight cases (flight_regimes.py) set, and why
 NOT_VARIED = {
-    'mass': 'rigid-body constant of the cf2x model, read by the free-flight integration the goldens cover',
-    'inertia': 'derived from the collision box in both models (PhysicsParams.inertia_diag), not a free setting',
-    'lin_damping': 'free-flight dynamics, covered by the free-flight goldens; not read by the contact solve',
-    'ang_damping': 'free-flight dynamics, covered by the free-flight goldens; not read by the contact solve',
-    'max_coord_vel': 'velocity clamp before the solve; only binds above 100 m/s',
-    'gyro': 'free-flight dynamics, covered by the free-flight goldens; not read by the contact solve',
-    'ang_motion_threshold': 'integration cap of the attitude update, not read by the contact solve',
+    'inertia': 'derived from the mass and the collision box in both models (PhysicsParams.inertia_diag), not a free '
+               'setting; the mass case of flight_regimes.py sets it with the mass',
     'ground_z': 'scene geometry of plane.urdf, fixed by the reference world',
     'col_radius': 'cf2x collision cylinder, fixed by the reference model',
     'col_halfheight': 'cf2x collision cylinder, fixed by the reference model',

@@ -1,6 +1,6 @@
 """Oracle-only checks behind test_gpu_physics_variants.py: every physics variant, in the start state the GPU tests
 use it in, moves the oracle's step far beyond the bar the GPU is held to (so a kernel that ignored the field would
-fail there), and every MrsPhysicsParams field is either varied or excused by name."""
+fail there), and every MrsPhysicsParams field is varied here or by the free-flight cases, or excused by name."""
 import dataclasses
 
 import numpy as np
@@ -15,10 +15,13 @@ SHAPES = [(12, 5), (8, 12), (67, 8), (10, 16), (4, 32), (6, 48), (2, 200)]
 
 
 def test_every_physics_field_is_varied_or_excused():
+    """varied by a contact variant here, by a free-flight case (flight_regimes.py), or excused by name"""
     from mrsgym_b200 import _abi
+    import flight_regimes as F
     fields = {f for f, _ in _abi.MrsPhysicsParams._fields_}
-    assert set(V.PHYS_FIELDS) | set(V.NOT_VARIED) == fields
-    assert not set(V.PHYS_FIELDS) & set(V.NOT_VARIED)
+    flight = set().union(*(set(f) for _, f, _ in F.CASES.values())) - set(F.TOP_LEVEL)
+    assert set(V.PHYS_FIELDS) | flight | set(V.NOT_VARIED) == fields
+    assert not (set(V.PHYS_FIELDS) | flight) & set(V.NOT_VARIED)
     oracle_fields = {f.name for f in dataclasses.fields(bm.PhysicsParams)}
     assert set(V.PHYS_FIELDS.values()) <= oracle_fields
     varied = set()

@@ -23,9 +23,6 @@ from oracle import spec
 
 pytestmark = pytest.mark.gpu
 
-REL = 1e-4
-FLOOR = dict(pos=5e-7, vel=5e-7, angvel=1e-5, quat=3e-7)
-
 
 def _swarm(E, N, mode, K=0, comm_range=float('inf'), layout=None, **kw):
     import mrsgym_b200 as M
@@ -35,26 +32,6 @@ def _swarm(E, N, mode, K=0, comm_range=float('inf'), layout=None, **kw):
 
 def _dev(a):
     return torch.from_numpy(np.ascontiguousarray(a)).cuda()
-
-
-def _check_delta(tag, s0, g1, r1):
-    """one-step deltas, GPU vs oracle, both measured from the common start state s0"""
-    worst = {}
-    for k in ('pos', 'vel', 'angvel', 'quat'):
-        base = s0[k].astype(np.float64)
-        dg, dr = g1[k] - base, r1[k] - base
-        if k == 'quat':       # q and -q are the same rotation
-            flip = np.sum(g1[k] * r1[k], axis=-1, keepdims=True) < 0
-            dg = np.where(flip, -g1[k], g1[k]) - base
-        err = np.abs(dg - dr)
-        floor = FLOOR[k]
-        if k == 'pos':     # one float32 ulp of the stored coordinate (5e-7 m up to 8 m, 1e-6 m up to 16 m, ...)
-            floor = np.maximum(floor, np.spacing(np.abs(g1[k]).astype(np.float32)).astype(np.float64))
-        tol = REL * np.abs(dr) + floor
-        worst[k] = float(np.max(err / tol))
-        assert np.all(err <= tol), '%s: %s delta off by %.3g x tolerance (max err %.3g)' % (
-            tag, k, worst[k], err.max())
-    return worst
 
 
 # ------------------------------------------------------------------------------ adjacency
@@ -110,7 +87,7 @@ def test_one_step_delta_vs_oracle(mode, E, N):
     g1 = H.read_state(sw)
     ref = H.make_spec(E, N, mode, 1, 1.5, st)
     Xr, Ar = ref.step(act[0])
-    _check_delta('%s E%d N%d' % (mode, E, N), st, g1, H.spec_state(ref))
+    H.check_delta('%s E%d N%d' % (mode, E, N), st, g1, H.spec_state(ref))
     # observation written by the same launch: X = float32 state, A = adjacency of ITS positions
     X = sw.X_window()[0].cpu().numpy()
     np.testing.assert_array_equal(X[..., :3], g1['pos'].astype(np.float32))
@@ -136,7 +113,7 @@ def test_controller_state_carries_over_steps(mode):
         ref.set_state(pos=s0['pos'], quat=s0['quat'], vel=s0['vel'], angvel=s0['angvel'])
         sw.step(_dev(act[t]))
         ref.step(act[t])
-        _check_delta('%s step %d' % (mode, t), {k: v.astype(np.float32) for k, v in s0.items()}, H.read_state(sw),
+        H.check_delta('%s step %d' % (mode, t), {k: v.astype(np.float32) for k, v in s0.items()}, H.read_state(sw),
                      H.spec_state(ref))
 
 
@@ -150,7 +127,7 @@ def test_no_action_step_is_free_fall():
     sw.step(None)
     ref = H.make_spec(E, N, 'set_speeds', 0, float('inf'), st)
     ref.step(None)
-    _check_delta('no action', st, H.read_state(sw), H.spec_state(ref))
+    H.check_delta('no action', st, H.read_state(sw), H.spec_state(ref))
 
 
 # ------------------------------------------------------------------------------ contact
@@ -569,7 +546,7 @@ def test_full_size_c4_single_env_4096_agents():
     sw.step(_dev(act[0]))
     ref = H.make_spec(E, N, 'set_force', 0, R, st)
     ref.step(act[0])
-    _check_delta('c4', st, H.read_state(sw), H.spec_state(ref))
+    H.check_delta('c4', st, H.read_state(sw), H.spec_state(ref))
     X = sw.X_window()[0].cpu().numpy()
     A = sw.A_window()[0].cpu()
     assert int((A != H.torch_cpu_adjacency(X[..., :3], R)).sum()) == 0
@@ -596,7 +573,7 @@ def test_ragged_shapes_one_step(E, N):
     sw.step(_dev(act[0]))
     ref = H.make_spec(E, N, 'set_target_vel', 1, 1.5, st)
     ref.step(act[0])
-    _check_delta('ragged E%d N%d' % (E, N), st, H.read_state(sw), H.spec_state(ref))
+    H.check_delta('ragged E%d N%d' % (E, N), st, H.read_state(sw), H.spec_state(ref))
     X = sw.X_window()[0].cpu().numpy()
     np.testing.assert_array_equal(sw.A_window()[0].cpu().numpy(), spec.adjacency(X[..., :3], 1.5))
 
