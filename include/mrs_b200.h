@@ -42,7 +42,7 @@
 extern "C" {
 #endif
 
-#define MRS_ABI_VERSION 4
+#define MRS_ABI_VERSION 5
 #define MRS_STATE_PLANES 13
 #define MRS_CTRL_PLANES 18
 #define MRS_STATS_SLOTS 8
@@ -287,6 +287,40 @@ int mrs_pack_adjacency(const MrsConfig* cfg, const float* A, unsigned int* bits,
 int mrs_spawn(const MrsConfig* cfg, const MrsBuffers* bufs, const unsigned char* env_mask,
               unsigned long long seed, unsigned long long env_offset, float z_lo, float z_hi, float xy_radius, float xy_sigma, float yaw_lo,
               float yaw_hi, int max_rounds, unsigned int* failed_envs, void* stream);
+
+/* Closed-loop episode bookkeeping and auto-reset, once per step after the step: the tail of the loop of
+ * examples/simulating_data/helper/DataGenerator.py:8-48 (done -> masked reset -> calc_Ak) without a host decision,
+ * so that a closed loop can be captured in a CUDA graph.  For every env e, with n = env_steps[e] (steps since its
+ * last reset, counted BEFORE this step's increment, as MRS.done_fn sees it):
+ *   done = (done_in && done_in[e]) || (max_timesteps >= 0 && n >= max_timesteps)
+ *          || (episode_length > 0 && n + 1 >= episode_length);
+ *   done_out[e] = done.
+ * A done env starts episode episode[e] + 1: its start state is redrawn with the default distribution and the
+ * 2*AGENT_RADIUS rejection rule of mrs_spawn (at most max_rounds rounds; an env still flagged keeps its last draw and
+ * counts once in *failed_envs), keyed by (seed, env_offset + e, episode[e] + 1) with ONE key packing for every N --
+ * the draw depends neither on E, the launch shape nor the step the reset falls on; velocities and angular
+ * velocities become zero, the PID planes are left alone (reference quirk, SURVEY.md §3.3); X0 (state_layout) is
+ * written into the K+1 X window slots (slot_x + k) mod L, A0 (the dense adjacency of the new positions, the
+ * predicate of mrs_adjacency) into slot_a and zeros into the K older A slots (slot_a + k) mod L; episode[e] += 1,
+ * env_steps[e] = 0.  Any other env only gets env_steps[e] += 1: no byte of its state, PID planes or tapes changes.
+ * A warp per env for N <= 32, a CTA per env above.  Stream-ordered, no host synchronisation, capturable.
+ * MRS_ERR_ARG: missing env_steps / episode / done_out, an X tape with MRS_X_NONE, a slot outside [0, L);
+ * MRS_ERR_UNSUPPORTED: E*N does not fit 32-bit slot indices. */
+typedef struct {
+    unsigned long long seed, env_offset;     /* as mrs_spawn */
+    float z_lo, z_hi, xy_radius, xy_sigma, yaw_lo, yaw_hi;
+    int max_rounds;
+    int episode_length;                      /* 0 = no limit */
+    int max_timesteps;                       /* MRS.MAX_TIMESTEPS as the default done_fn sees it; <0 = inf */
+} MrsAutoResetArgs;
+
+int mrs_autoreset(const MrsConfig* cfg, const MrsBuffers* bufs, const MrsAutoResetArgs* a,
+                  const unsigned char* done_in,   /* device [E] or NULL: the user's done_fn result */
+                  int* env_steps,                 /* device [E], steps since the env's last reset, in/out */
+                  unsigned* episode,              /* device [E], episodes started per env, in/out */
+                  unsigned char* done_out,        /* device [E]: the dataset's done[t] */
+                  int slot_x, int slot_a,         /* newest X / A slots; window slots are (slot + k) mod L */
+                  unsigned* failed_envs, void* stream);
 
 /* Analytic sensors on the primitives of the 'simple' world (ground box top at ground_z, agents as
  * phys.contact_radius spheres: the contact geometry of the step's pair rows; phys.agent_radius is only

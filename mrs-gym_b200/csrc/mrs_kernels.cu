@@ -212,33 +212,29 @@ __device__ __forceinline__ unsigned long long splitmix64(unsigned long long x) {
 }
 __device__ __forceinline__ float u01(unsigned long long h) { return ((h >> 40) + 0.5f) * (1.0f / 16777216.0f); }
 
-__global__ void __launch_bounds__(128)
-spawn_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const SpawnArgs sp,
-             const unsigned char* __restrict__ mask, unsigned* __restrict__ failed) {
-    const int lane = threadIdx.x & 31;
-    const int e = blockIdx.x * 4 + (threadIdx.x >> 5);
-    if (e >= c.E) return;
-    if (mask && !mask[e]) return;
-    const int N = c.N;
-    const unsigned S = (unsigned)c.E * (unsigned)N;
+// One start position from draw key `key`: Box-Muller xy pulled onto the disc, z uniform (mrs_spawn, mrs_autoreset).
+__device__ __forceinline__ void spawn_draw(unsigned long long key, const SpawnArgs& sp, float& x, float& y, float& z) {
+    const float u1 = u01(key), u2 = u01(splitmix64(key)), u3 = u01(splitmix64(key ^ 0x5851F42D4C957F2Dull));
+    const float r = sp.xy_sigma * sqrtf(-2.f * logf(u1));          // Box-Muller
+    float sn, cs;
+    sincosf(6.28318530717958647692f * u2, &sn, &cs);
+    x = r * cs; y = r * sn;
+    const float mag = fmaxf(sqrtf(x * x + y * y), sp.xy_radius);     // SphereTransform(within=True)
+    x = x / mag * sp.xy_radius; y = y / mag * sp.xy_radius;
+    z = sp.z_lo + (sp.z_hi - sp.z_lo) * u3;
+}
+
+// Rejection rounds of one env on one warp (N <= 32, lane = agent): every flagged lane (all of them in round 0) draws
+// with key_of(round), then a lane is flagged iff a lower lane lies closer than 2*AGENT_RADIUS.  Returns the rounds
+// run; max_rounds means the env did not converge.
+template <class KeyOf>
+__device__ __forceinline__ int spawn_warp_rounds(const SpawnArgs& sp, int N, int lane, float lim2, KeyOf key_of,
+                                                 float& x, float& y, float& z) {
     const bool valid = lane < N;
-    const float lim2 = 4.f * c.phys.agent_radius * c.phys.agent_radius;
-    float x = 0.f, y = 0.f, z = 0.f;
     bool redraw = true;
     int round = 0;
     for (; round < sp.max_rounds; ++round) {
-        if (redraw && valid) {
-            const unsigned long long ge = sp.env_offset + (unsigned long long)e;      // global env index: shards draw different envs
-            const unsigned long long key = splitmix64(sp.seed ^ splitmix64((ge << 20) ^ ((unsigned long long)lane << 12) ^ (unsigned long long)round));
-            const float u1 = u01(key), u2 = u01(splitmix64(key)), u3 = u01(splitmix64(key ^ 0x5851F42D4C957F2Dull));
-            const float r = sp.xy_sigma * sqrtf(-2.f * logf(u1));          // Box-Muller
-            float sn, cs;
-            sincosf(6.28318530717958647692f * u2, &sn, &cs);
-            x = r * cs; y = r * sn;
-            const float mag = fmaxf(sqrtf(x * x + y * y), sp.xy_radius);     // SphereTransform(within=True)
-            x = x / mag * sp.xy_radius; y = y / mag * sp.xy_radius;
-            z = sp.z_lo + (sp.z_hi - sp.z_lo) * u3;
-        }
+        if (redraw && valid) spawn_draw(key_of(round), sp, x, y, z);
         bool hit = false;
         for (int j = 0; j < N; ++j) {
             const float xj = __shfl_sync(kFull32, x, j), yj = __shfl_sync(kFull32, y, j), zj = __shfl_sync(kFull32, z, j);
@@ -248,18 +244,40 @@ spawn_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const Spaw
         redraw = hit;
         if (!__any_sync(kFull32, hit)) break;
     }
+    return round;
+}
+
+// Attitude and rates of a fresh start: yaw only (roll = pitch = 0), velocities zero.  st: the agent's plane-0 entry.
+__device__ __forceinline__ void spawn_write_rest(float* st, size_t S, float yaw) {
+    float sy, cy;
+    sincosf(0.5f * yaw, &sy, &cy);
+    st[3 * S] = 0.f; st[4 * S] = 0.f; st[5 * S] = sy; st[6 * S] = cy;
+#pragma unroll
+    for (int p = 7; p < 13; ++p) st[p * S] = 0.f;
+}
+
+__global__ void __launch_bounds__(128)
+spawn_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const SpawnArgs sp,
+             const unsigned char* __restrict__ mask, unsigned* __restrict__ failed) {
+    const int lane = threadIdx.x & 31;
+    const int e = blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (e >= c.E) return;
+    if (mask && !mask[e]) return;
+    const int N = c.N;
+    const unsigned S = (unsigned)c.E * (unsigned)N;
+    const float lim2 = 4.f * c.phys.agent_radius * c.phys.agent_radius;
+    const unsigned long long ge = sp.env_offset + (unsigned long long)e;      // global env index: shards draw different envs
+    float x = 0.f, y = 0.f, z = 0.f;
+    const int round = spawn_warp_rounds(sp, N, lane, lim2, [&](int r) {
+        return splitmix64(sp.seed ^ splitmix64((ge << 20) ^ ((unsigned long long)lane << 12) ^ (unsigned long long)r));
+    }, x, y, z);
     if (round >= sp.max_rounds && lane == 0 && failed) atomicAdd(failed, 1u);
-    if (!valid) return;
+    if (lane >= N) return;
     const unsigned s = (unsigned)e * (unsigned)N + (unsigned)lane;
     float* st = b.state;
     st[0 * (size_t)S + s] = x; st[1 * (size_t)S + s] = y; st[2 * (size_t)S + s] = z;
     const unsigned long long ky = splitmix64(sp.seed ^ splitmix64(0xA5A5A5A5ull ^ ((sp.env_offset + (unsigned long long)e) << 20) ^ ((unsigned long long)lane << 12)));
-    const float yaw = sp.yaw_lo + (sp.yaw_hi - sp.yaw_lo) * u01(ky);
-    float sy, cy;
-    sincosf(0.5f * yaw, &sy, &cy);
-    st[3 * (size_t)S + s] = 0.f; st[4 * (size_t)S + s] = 0.f; st[5 * (size_t)S + s] = sy; st[6 * (size_t)S + s] = cy;
-#pragma unroll
-    for (int p = 7; p < 13; ++p) st[p * (size_t)S + s] = 0.f;
+    spawn_write_rest(st + s, S, sp.yaw_lo + (sp.yaw_hi - sp.yaw_lo) * u01(ky));
 }
 
 // Wide form (N > 32): one CTA per env, the same draws and the same rejection rule, stated per agent: in round r
@@ -278,37 +296,19 @@ __device__ __forceinline__ unsigned long long spawn_wide_key(unsigned long long 
     return splitmix64(seed ^ splitmix64(env_hash ^ (((unsigned long long)agent << 32) | round)));
 }
 
-__global__ void __launch_bounds__(1024)
-spawn_wide_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const SpawnArgs sp,
-                  const unsigned char* __restrict__ mask, unsigned* __restrict__ failed) {
-    extern __shared__ unsigned spawn_bits[];
-    const unsigned e = blockIdx.x;
-    if (mask && !mask[e]) return;
-    const int N = c.N;
+// The rejection rounds of one env on one CTA (see above); `spawn_bits` holds the two masks.  Returns the rounds run.
+__device__ __forceinline__ int spawn_cta_rounds(const SpawnArgs& sp, int N, float lim2, unsigned long long env_hash,
+                                                unsigned* spawn_bits, float* px, float* py, float* pz) {
     const int W = (N + 31) / 32;
     unsigned* moved = spawn_bits;          // agents that draw in this round
     unsigned* flag = spawn_bits + W;       // agents flagged by this round's test
-    const size_t S = (size_t)c.E * (size_t)N;
-    float* px = b.state + (size_t)e * N;
-    float* py = px + S;
-    float* pz = py + S;
-    const float lim2 = 4.f * c.phys.agent_radius * c.phys.agent_radius;
-    const unsigned long long env_hash = splitmix64(sp.env_offset + (unsigned long long)e);
     for (int w = threadIdx.x; w < W; w += blockDim.x) moved[w] = (w == W - 1 && (N & 31)) ? (1u << (N & 31)) - 1u : kFull32;
     __syncthreads();
     int round = 0;
     for (; round < sp.max_rounds; ++round) {
         for (int i = threadIdx.x; i < N; i += blockDim.x) {
             if (!((moved[i >> 5] >> (i & 31)) & 1u)) continue;
-            const unsigned long long key = spawn_wide_key(sp.seed, env_hash, (unsigned)i, (unsigned)round);
-            const float u1 = u01(key), u2 = u01(splitmix64(key)), u3 = u01(splitmix64(key ^ 0x5851F42D4C957F2Dull));
-            const float r = sp.xy_sigma * sqrtf(-2.f * logf(u1));          // Box-Muller
-            float sn, cs;
-            sincosf(6.28318530717958647692f * u2, &sn, &cs);
-            float x = r * cs, y = r * sn;
-            const float mag = fmaxf(sqrtf(x * x + y * y), sp.xy_radius);     // SphereTransform(within=True)
-            x = x / mag * sp.xy_radius; y = y / mag * sp.xy_radius;
-            px[i] = x; py[i] = y; pz[i] = sp.z_lo + (sp.z_hi - sp.z_lo) * u3;
+            spawn_draw(spawn_wide_key(sp.seed, env_hash, (unsigned)i, (unsigned)round), sp, px[i], py[i], pz[i]);
         }
         for (int w = threadIdx.x; w < W; w += blockDim.x) flag[w] = 0u;
         __syncthreads();                   // this round's positions and the cleared flags are visible to the CTA
@@ -338,17 +338,42 @@ spawn_wide_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const
         }
         if (!__syncthreads_or(any)) break;
     }
-    if (round >= sp.max_rounds && threadIdx.x == 0 && failed) atomicAdd(failed, 1u);
+    return round;
+}
+
+__global__ void __launch_bounds__(1024)
+spawn_wide_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const SpawnArgs sp,
+                  const unsigned char* __restrict__ mask, unsigned* __restrict__ failed) {
+    extern __shared__ unsigned spawn_bits[];
+    const unsigned e = blockIdx.x;
+    if (mask && !mask[e]) return;
+    const int N = c.N;
+    const size_t S = (size_t)c.E * (size_t)N;
     float* st = b.state + (size_t)e * N;
+    const float lim2 = 4.f * c.phys.agent_radius * c.phys.agent_radius;
+    const unsigned long long env_hash = splitmix64(sp.env_offset + (unsigned long long)e);
+    const int round = spawn_cta_rounds(sp, N, lim2, env_hash, spawn_bits, st, st + S, st + 2 * S);
+    if (round >= sp.max_rounds && threadIdx.x == 0 && failed) atomicAdd(failed, 1u);
     for (int i = threadIdx.x; i < N; i += blockDim.x) {
         const unsigned long long ky = spawn_wide_key(sp.seed, env_hash, (unsigned)i, 0xFFFFFFFFu);
-        const float yaw = sp.yaw_lo + (sp.yaw_hi - sp.yaw_lo) * u01(ky);
-        float sy, cy;
-        sincosf(0.5f * yaw, &sy, &cy);
-        st[3 * S + i] = 0.f; st[4 * S + i] = 0.f; st[5 * S + i] = sy; st[6 * S + i] = cy;
-#pragma unroll
-        for (int p = 7; p < 13; ++p) st[p * S + i] = 0.f;
+        spawn_write_rest(st + i, S, sp.yaw_lo + (sp.yaw_hi - sp.yaw_lo) * u01(ky));
     }
+}
+
+// Raises `kernel`'s dynamic shared-memory limit to `smem` when that is above the default 48 KB (once per size and
+// device; configured[dev] keeps the largest size set so far).
+template <class Kernel>
+static int ensure_dynamic_smem(Kernel kernel, size_t smem, size_t* configured) {
+    int dev = 0, optin = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return MRS_ERR_CUDA;
+    if (smem > configured[dev] && smem > 48 * 1024) {
+        if (cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess) return MRS_ERR_CUDA;
+        if (smem > (size_t)optin) return MRS_ERR_UNSUPPORTED;
+        if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return MRS_ERR_CUDA;
+        configured[dev] = smem;
+    }
+    return MRS_OK;
 }
 
 static int launch_spawn_wide(const MrsConfig& c, const MrsBuffers& b, const SpawnArgs& sp, const unsigned char* mask,
@@ -358,17 +383,152 @@ static int launch_spawn_wide(const MrsConfig& c, const MrsBuffers& b, const Spaw
     const size_t smem = 2 * (size_t)((c.N + 31) / 32) * sizeof(unsigned);
     // the two bit masks grow with N: raise the kernel's dynamic shared-memory limit to the largest size asked for
     static size_t configured[64] = {};
-    int dev = 0, optin = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return MRS_ERR_CUDA;
-    if (smem > configured[dev] && smem > 48 * 1024) {
-        if (cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess) return MRS_ERR_CUDA;
-        if (smem > (size_t)optin) return MRS_ERR_UNSUPPORTED;
-        if (cudaFuncSetAttribute(spawn_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MRS_ERR_CUDA;
-        configured[dev] = smem;
-    }
+    const int rc = ensure_dynamic_smem(spawn_wide_kernel, smem, configured);
+    if (rc) return rc;
     spawn_wide_kernel<<<(unsigned)c.E, (unsigned)threads, smem, st>>>(c, b, sp, mask, failed);
     return last_error();
+}
+
+// ------------------------------------------------------------------------------ auto-reset (mrs_autoreset)
+// Episode bookkeeping of a closed loop plus the masked reset of the envs whose episode ended (header: the done rule
+// and what a reset writes).  The draws are those of mrs_spawn -- spawn_draw and the same rejection rule -- under
+// ONE key packing for every N: spawn_wide_key (agent, round) under a per-(env, episode) hash, so a reset depends on
+// (seed, env_offset + e, episode) only.
+struct AutoResetArgs {
+    SpawnArgs sp;
+    int episode_length, max_timesteps;
+    int slot_x, slot_a;
+    float s_max;
+    int comm_inf;
+};
+
+__device__ __forceinline__ unsigned long long autoreset_env_hash(unsigned long long global_env, unsigned episode) {
+    return splitmix64(splitmix64(global_env) ^ splitmix64(0xD1B54A32D192ED03ull ^ (unsigned long long)episode));
+}
+
+// the done rule: done_fn / MAX_TIMESTEPS see the count before the step's increment, episode_length the count after
+__device__ __forceinline__ bool autoreset_done(const AutoResetArgs& a, const unsigned char* done_in, unsigned e, int n) {
+    return (done_in && done_in[e]) || (a.max_timesteps >= 0 && n >= a.max_timesteps) ||
+           (a.episode_length > 0 && n + 1 >= a.episode_length);
+}
+
+// X0 of agent slot s (position, yaw-only attitude, zero rates: what spawn_write_rest stored) into the K+1 X window
+// slots.  Built from registers, not re-read from the state planes this kernel has just written.
+__device__ __forceinline__ void autoreset_write_X(const MrsConfig& c, const MrsBuffers& b, const AutoResetArgs& a,
+                                                  unsigned S, unsigned s, float x, float y, float z, float yaw) {
+    if (!b.X_tape) return;
+    Agent ag;
+    ag.px = x; ag.py = y; ag.pz = z;
+    float sy, cy;
+    sincosf(0.5f * yaw, &sy, &cy);
+    ag.qx = 0.f; ag.qy = 0.f; ag.qz = sy; ag.qw = cy;
+    ag.vx = ag.vy = ag.vz = 0.f;
+    ag.wx = ag.wy = ag.wz = 0.f;
+    const size_t slot_elems = (size_t)S * (size_t)state_dim(c.state_layout);
+    for (int k = 0; k <= c.K; ++k)
+        write_X(b.X_tape + (size_t)((a.slot_x + k) % c.L) * slot_elems, c.state_layout, s, ag);
+}
+
+__device__ __forceinline__ float autoreset_adjacency(const AutoResetArgs& a, int i, int j, float xi, float yi, float zi,
+                                                     float xj, float yj, float zj) {
+    return (i == j) ? 0.f : (a.comm_inf ? 1.f : adjacency_pair(xi, yi, zi, xj, yj, zj, a.s_max));
+}
+
+// N <= 32: a warp per env, lane = agent, 4 envs per CTA
+__global__ void __launch_bounds__(128)
+autoreset_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const AutoResetArgs a,
+                 const unsigned char* __restrict__ done_in, int* __restrict__ env_steps, unsigned* __restrict__ episode,
+                 unsigned char* __restrict__ done_out, unsigned* __restrict__ failed) {
+    const int lane = threadIdx.x & 31;
+    const unsigned e = blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (e >= (unsigned)c.E) return;
+    const int n = env_steps[e];
+    const bool done = autoreset_done(a, done_in, e, n);
+    const unsigned ep = episode[e] + 1u;
+    __syncwarp();
+    if (!done) {
+        if (lane == 0) { env_steps[e] = n + 1; done_out[e] = 0; }
+        return;
+    }
+    const int N = c.N;
+    const unsigned S = (unsigned)c.E * (unsigned)N;
+    const float lim2 = 4.f * c.phys.agent_radius * c.phys.agent_radius;
+    const unsigned long long env_hash = autoreset_env_hash(a.sp.env_offset + e, ep);
+    float x = 0.f, y = 0.f, z = 0.f;
+    const int round = spawn_warp_rounds(a.sp, N, lane, lim2, [&](int r) {
+        return spawn_wide_key(a.sp.seed, env_hash, (unsigned)lane, (unsigned)r);
+    }, x, y, z);
+    if (lane == 0) {
+        if (round >= a.sp.max_rounds && failed) atomicAdd(failed, 1u);
+        episode[e] = ep; env_steps[e] = 0; done_out[e] = 1;
+    }
+    const unsigned s = e * (unsigned)N + (unsigned)lane;
+    if (lane < N) {
+        float* st = b.state + s;
+        st[0] = x; st[(size_t)S] = y; st[2 * (size_t)S] = z;
+        const float yaw = a.sp.yaw_lo + (a.sp.yaw_hi - a.sp.yaw_lo) * u01(spawn_wide_key(a.sp.seed, env_hash, (unsigned)lane, 0xFFFFFFFFu));
+        spawn_write_rest(st, S, yaw);
+        autoreset_write_X(c, b, a, S, s, x, y, z, yaw);
+    }
+    if (!b.A_tape) return;
+    const unsigned NN = (unsigned)(N * N);
+    const size_t slot_elems = (size_t)S * (size_t)N;
+    float* A0 = b.A_tape + (size_t)a.slot_a * slot_elems + (size_t)e * NN;
+    for (unsigned base = 0; base < NN; base += 32) {          // whole warp: the shuffles need every lane
+        const unsigned idx = base + (unsigned)lane;
+        const int i = idx < NN ? (int)(idx / (unsigned)N) : 0, j = idx < NN ? (int)(idx % (unsigned)N) : 0;
+        const float xi = __shfl_sync(kFull32, x, i), yi = __shfl_sync(kFull32, y, i), zi = __shfl_sync(kFull32, z, i);
+        const float xj = __shfl_sync(kFull32, x, j), yj = __shfl_sync(kFull32, y, j), zj = __shfl_sync(kFull32, z, j);
+        if (idx < NN) A0[idx] = autoreset_adjacency(a, i, j, xi, yi, zi, xj, yj, zj);
+    }
+    for (int k = 1; k <= c.K; ++k) {
+        float* Ak = b.A_tape + (size_t)((a.slot_a + k) % c.L) * slot_elems + (size_t)e * NN;
+        for (unsigned idx = lane; idx < NN; idx += 32) Ak[idx] = 0.f;
+    }
+}
+
+// N > 32: a CTA per env, the rounds of spawn_wide_kernel; dynamic shared memory = its two masks
+__global__ void __launch_bounds__(1024)
+autoreset_wide_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const AutoResetArgs a,
+                      const unsigned char* __restrict__ done_in, int* __restrict__ env_steps, unsigned* __restrict__ episode,
+                      unsigned char* __restrict__ done_out, unsigned* __restrict__ failed) {
+    extern __shared__ unsigned spawn_bits[];
+    const unsigned e = blockIdx.x;
+    const int n = env_steps[e];
+    const bool done = autoreset_done(a, done_in, e, n);
+    const unsigned ep = episode[e] + 1u;
+    __syncthreads();                       // every thread has read the counters before thread 0 rewrites them
+    if (!done) {
+        if (threadIdx.x == 0) { env_steps[e] = n + 1; done_out[e] = 0; }
+        return;
+    }
+    const int N = c.N;
+    const size_t S = (size_t)c.E * (size_t)N;
+    float* st = b.state + (size_t)e * N;
+    const float lim2 = 4.f * c.phys.agent_radius * c.phys.agent_radius;
+    const unsigned long long env_hash = autoreset_env_hash(a.sp.env_offset + e, ep);
+    const int round = spawn_cta_rounds(a.sp, N, lim2, env_hash, spawn_bits, st, st + S, st + 2 * S);
+    if (threadIdx.x == 0) {
+        if (round >= a.sp.max_rounds && failed) atomicAdd(failed, 1u);
+        episode[e] = ep; env_steps[e] = 0; done_out[e] = 1;
+    }
+    for (int i = threadIdx.x; i < N; i += blockDim.x) {
+        const float yaw = a.sp.yaw_lo + (a.sp.yaw_hi - a.sp.yaw_lo) * u01(spawn_wide_key(a.sp.seed, env_hash, (unsigned)i, 0xFFFFFFFFu));
+        spawn_write_rest(st + i, S, yaw);
+        autoreset_write_X(c, b, a, (unsigned)S, e * (unsigned)N + (unsigned)i, st[i], st[S + i], st[2 * S + i], yaw);
+    }
+    if (!b.A_tape) return;
+    const size_t NN = (size_t)N * N;
+    const size_t slot_elems = S * (size_t)N;
+    float* A0 = b.A_tape + (size_t)a.slot_a * slot_elems + (size_t)e * NN;
+    for (size_t idx = threadIdx.x; idx < NN; idx += blockDim.x) {     // positions: this CTA's writes, before the last barrier
+        const int i = (int)(idx / (unsigned)N), j = (int)(idx % (unsigned)N);
+        A0[idx] = autoreset_adjacency(a, i, j, st[i], st[S + i], st[2 * S + i], st[j], st[S + j], st[2 * S + j]);
+    }
+    for (int k = 1; k <= c.K; ++k) {
+        float* Ak = b.A_tape + (size_t)((a.slot_a + k) % c.L) * slot_elems + (size_t)e * NN;
+        for (size_t idx = threadIdx.x; idx < NN; idx += blockDim.x) Ak[idx] = 0.f;
+    }
 }
 
 // ------------------------------------------------------------------------------ sensors (row f4)
@@ -1063,6 +1223,42 @@ int mrs_spawn(const MrsConfig* cfg, const MrsBuffers* bufs, const unsigned char*
     // a warp per env packs 4 envs into a CTA; past 32 agents an env takes a CTA of its own
     if (cfg->N > 32) return launch_spawn_wide(*cfg, *bufs, sp, env_mask, failed_envs, (cudaStream_t)stream);
     spawn_kernel<<<(unsigned)((cfg->E + 3) / 4), 128, 0, (cudaStream_t)stream>>>(*cfg, *bufs, sp, env_mask, failed_envs);
+    return last_error();
+}
+
+
+int mrs_autoreset(const MrsConfig* cfg, const MrsBuffers* bufs, const MrsAutoResetArgs* args, const unsigned char* done_in,
+                  int* env_steps, unsigned* episode, unsigned char* done_out, int slot_x, int slot_a, unsigned* failed_envs,
+                  void* stream) {
+    int rc = check_cfg(cfg);
+    if (rc) return rc;
+    if (!bufs || !bufs->state || !args || !env_steps || !episode || !done_out) return MRS_ERR_ARG;
+    if (!(args->z_hi >= args->z_lo) || !(args->xy_radius > 0.f) || !(args->xy_sigma > 0.f) || args->max_rounds <= 0)
+        return MRS_ERR_ARG;
+    if (bufs->X_tape && (cfg->state_layout == MRS_X_NONE || slot_x < 0 || slot_x >= cfg->L)) return MRS_ERR_ARG;
+    if (bufs->A_tape && (slot_a < 0 || slot_a >= cfg->L)) return MRS_ERR_ARG;
+    if ((size_t)cfg->E * (size_t)cfg->N > 0xffffffffull) return MRS_ERR_UNSUPPORTED;     // u32 slot indices
+    AutoResetArgs a;
+    a.sp.seed = args->seed; a.sp.env_offset = args->env_offset; a.sp.z_lo = args->z_lo; a.sp.z_hi = args->z_hi;
+    a.sp.xy_radius = args->xy_radius; a.sp.xy_sigma = args->xy_sigma; a.sp.yaw_lo = args->yaw_lo; a.sp.yaw_hi = args->yaw_hi;
+    a.sp.max_rounds = args->max_rounds;
+    a.episode_length = args->episode_length; a.max_timesteps = args->max_timesteps;
+    a.slot_x = slot_x; a.slot_a = slot_a;
+    const Derived d = make_derived(*cfg);         // s_max / comm_inf exactly as the step kernels derive them
+    a.s_max = d.s_max; a.comm_inf = d.comm_inf;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (cfg->N > 32) {
+        int threads = (cfg->N + 31) / 32 * 32;
+        if (threads > 1024) threads = 1024;
+        const size_t smem = 2 * (size_t)((cfg->N + 31) / 32) * sizeof(unsigned);
+        static size_t configured[64] = {};
+        if ((rc = ensure_dynamic_smem(autoreset_wide_kernel, smem, configured))) return rc;
+        autoreset_wide_kernel<<<(unsigned)cfg->E, (unsigned)threads, smem, st>>>(*cfg, *bufs, a, done_in, env_steps, episode,
+                                                                                 done_out, failed_envs);
+    } else {
+        autoreset_kernel<<<(unsigned)((cfg->E + 3) / 4), 128, 0, st>>>(*cfg, *bufs, a, done_in, env_steps, episode, done_out,
+                                                                      failed_envs);
+    }
     return last_error();
 }
 

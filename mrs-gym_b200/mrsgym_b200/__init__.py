@@ -12,7 +12,7 @@ from ._abi import MrsError
 from .core import Swarm, Neighbors, shard_range
 from .env import MRS, Environment, AgentBatch
 from .spawn import DefaultSpawn, sample_start_pos
-from .rollout import rollout, reynolds_policy, to_trainer_history, save_dataset
+from .rollout import rollout, reynolds_policy, to_trainer_history, save_dataset, ClosedLoopGraph
 from .wrappers import MRS_RLlib, MRS_RLlib_MultiAgent
 
 _REGISTRY = {'mrs-v0': MRS, 'mrs-rllib-v0': MRS_RLlib, 'mrs-rllib-multiagent-v0': MRS_RLlib_MultiAgent}

@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('MRS_B200_LIB') or os.path.join(_HERE, 'libmrs_b200.so')   # override: A/B builds
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 STATE_PLANES = 13
 CTRL_PLANES = 18
 STATS_SLOTS = 8
@@ -82,6 +82,12 @@ class MrsBuffers(C.Structure):
                 ('status', C.c_void_p), ('stats', C.c_void_p), ('sync', C.c_void_p)]
 
 
+class MrsAutoResetArgs(C.Structure):
+    _fields_ = [('seed', C.c_ulonglong), ('env_offset', C.c_ulonglong),
+                ('z_lo', f), ('z_hi', f), ('xy_radius', f), ('xy_sigma', f), ('yaw_lo', f), ('yaw_hi', f),
+                ('max_rounds', C.c_int), ('episode_length', C.c_int), ('max_timesteps', C.c_int)]
+
+
 class MrsError(RuntimeError):
     pass
 
@@ -116,6 +122,8 @@ _SIGNATURES = {
                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     'mrs_spawn': (C.c_int, [C.POINTER(MrsConfig), C.POINTER(MrsBuffers), C.c_void_p, C.c_ulonglong, C.c_ulonglong, C.c_float, C.c_float,
                             C.c_float, C.c_float, C.c_float, C.c_float, C.c_int, C.c_void_p, C.c_void_p]),
+    'mrs_autoreset': (C.c_int, [C.POINTER(MrsConfig), C.POINTER(MrsBuffers), C.POINTER(MrsAutoResetArgs), C.c_void_p,
+                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     'mrs_proximity': (C.c_int, [C.POINTER(MrsConfig), C.POINTER(MrsBuffers), C.c_float, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.c_void_p]),
     'mrs_raycast': (C.c_int, [C.POINTER(MrsConfig), C.POINTER(MrsBuffers), C.c_void_p, C.c_int, C.POINTER(C.c_float),

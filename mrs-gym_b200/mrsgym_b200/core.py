@@ -581,6 +581,32 @@ class Swarm:
         self.launches += 1
         return failed
 
+    def autoreset(self, seed, env_steps, episode, done_out, done_in=None, slot_x=None, slot_a=None, z=(1.0, 3.0),
+                  xy_radius=1.0, xy_sigma=1.0, yaw=(-math.pi / 2, math.pi / 2), max_rounds=256, env_offset=0,
+                  episode_length=0, max_timesteps=-1, failed=None):
+        """mrs_autoreset: the per-step episode bookkeeping of a closed loop, after the step.  env_steps (int32 [E]) and
+        episode (int32 [E], read as unsigned) are device counters updated in place; done_out (uint8 / bool [E]) receives
+        done[t]; done_in (bool / uint8 [E] or None) is the done_fn result.  Done envs are redrawn with the default start
+        distribution keyed by (seed, env_offset + e, episode + 1), their K+1 X window becomes X0 and their A window
+        A0 followed by K zero slices; the other envs only count the step.  slot_x / slot_a: the newest slots of the
+        windows (default: the current heads).  failed (int32 [1], added to): envs whose rejection sampling did not
+        converge.  Stream-ordered and capturable."""
+        for t, what in ((env_steps, 'env_steps'), (episode, 'episode')):
+            if t.dtype != torch.int32 or not t.is_contiguous() or t.numel() != self.E or t.device != self.device:
+                raise ValueError('%s must be a contiguous int32 [%d] tensor on %s' % (what, self.E, self.device))
+        if done_out.dtype not in (torch.uint8, torch.bool) or not done_out.is_contiguous() or done_out.numel() != self.E:
+            raise ValueError('done_out must be a contiguous uint8 / bool [%d] tensor' % self.E)
+        if done_in is not None and (done_in.dtype not in (torch.uint8, torch.bool) or not done_in.is_contiguous()
+                                    or done_in.numel() != self.E):
+            raise ValueError('done_in must be a contiguous uint8 / bool [%d] tensor' % self.E)
+        a = _abi.MrsAutoResetArgs(int(seed), int(env_offset), float(z[0]), float(z[1]), float(xy_radius), float(xy_sigma),
+                                  float(yaw[0]), float(yaw[1]), int(max_rounds), int(episode_length), int(max_timesteps))
+        _abi.check(self.lib.mrs_autoreset(self._cfg_ref, self._bufs_ref, C.byref(a), _ptr(done_in), _ptr(env_steps),
+                                          _ptr(episode), _ptr(done_out), self.hx if slot_x is None else int(slot_x),
+                                          self.ha if slot_a is None else int(slot_a), _ptr(failed), self._stream()),
+                   'mrs_autoreset')
+        self.launches += 1
+
     def set_quat(self, quat):
         """Exact quaternion upload (xyzw), bypassing the euler conversion (tests / checkpoints)."""
         q = torch.as_tensor(quat, dtype=torch.float32).to(self.device).reshape(self.S, 4)

@@ -166,6 +166,16 @@ class _Sim:
         pass
 
 
+def _zero_reward(**kwargs):
+    """Default reward_fn (MRS.py:37): 0."""
+    return 0.0
+
+
+def _no_info(**kwargs):
+    """Default info_fn (MRS.py:40): no extra info."""
+    return {}
+
+
 class MRS:
     metadata = {'render.modes': ['headless', 'bullet']}
 
@@ -199,11 +209,11 @@ class MRS:
         if env != 'simple':
             raise NotImplementedError("only the 'simple' world (N x cf2x + ground plane, EnvCreator.py:7-13) is in scope")
         self.state_fn = state_fn
-        self.reward_fn = reward_fn if (reward_fn is not None) else (lambda **kwargs: 0.0)
+        self.reward_fn = reward_fn if (reward_fn is not None) else _zero_reward
         # default done: steps since the last reset >= MAX_TIMESTEPS (MRS.py:39); batched: per env ([E] bool tensor,
         # a masked reset restarts the count of the selected envs only)
         self.done_fn = done_fn if (done_fn is not None) else self._default_done
-        self.info_fn = info_fn if (info_fn is not None) else (lambda **kwargs: {})
+        self.info_fn = info_fn if (info_fn is not None) else _no_info
         self.update_fn = update_fn
         self.start_fn = start_fn
         self.sim = _Sim(**kwargs)
@@ -241,6 +251,12 @@ class MRS:
         self._steps_total = 0
         self._steps_at_reset = torch.zeros(self.N_ENVS, dtype=torch.int64, device=self.swarm.device)
         self._uniform_reset = True      # no masked reset since the last full one: env_steps is the same for all envs
+        # rollout(graph=True): the graph's device step counter, which env_steps reports while the graph's body runs,
+        # the index of every env's current episode (advanced by the on-device auto-reset, the key of its draws) and
+        # the captured closed loops of this env
+        self._dev_steps = None
+        self.episode = torch.zeros(self.N_ENVS, dtype=torch.int32, device=self.swarm.device)
+        self._graphs = {}
         self._done_const = {}
         self.steps_since_reset = 0
         self.last_action = None
@@ -318,6 +334,8 @@ class MRS:
     @property
     def env_steps(self):
         """[E] int64: steps since each env's last (masked) reset."""
+        if self._dev_steps is not None:          # inside the body of rollout(graph=True): the device counter
+            return self._dev_steps.long()
         return self._steps_total - self._steps_at_reset
 
     # ------------------------------------------------------------------ observation windows
