@@ -326,13 +326,20 @@ int mrs_autoreset(const MrsConfig* cfg, const MrsBuffers* bufs, const MrsAutoRes
  * phys.contact_radius spheres: the contact geometry of the step's pair rows; phys.agent_radius is only
  * the spawn separation), for all agents of all envs at once.
  * mrs_proximity: per agent the gap to the nearest other agent (centre distance - 2*contact_radius) and
- * its index, the gap of the collision cylinder to the ground, and collision = any gap < threshold
- * (the reference uses 0.04).  Any output pointer may be NULL.  Device arrays of E*N elements.
+ * its index (the lowest index among equal distances; -1 and an infinite gap when N == 1), the gap of the
+ * collision cylinder to the ground, and collision = any gap < threshold (strict; the reference uses 0.04).  The
+ * ground gap is that of the lowest of the four rim points (+-col_radius, 0, cz), (0, +-col_radius, cz) that the
+ * step's ground rows use: z - col_radius*max(|R20|,|R21|) - col_halfheight*|R22| - col_margin - ground_z.
+ * Any output pointer may be NULL.  Device arrays of E*N elements.
  * Replaces Object.collision / get_dist / get_contact_points distances (Object.py:98-140).
  * mrs_raycast: n_rays rays per agent, directions device float[n_rays][3] in the body frame
  * (body_frame != 0) or the world frame, start = position + R * offset3 (HOST float[3], may be NULL);
  * hit_dist float[E*N][n_rays] (inf = nothing within range), hit_id int[E*N][n_rays]: -1 none,
- * N = ground, j = agent j of the same env.  Replaces Object.raycast (Object.py:143-174). */
+ * N = ground, j = agent j of the same env; the first hit at t < range wins, ties go to the ground, then the
+ * lowest index.  A direction counts by its orientation only: any finite nonzero magnitude (denormal to FLT_MAX)
+ * gives the result of its unit vector; a zero direction or one with a NaN or infinite component hits nothing
+ * (-1 / inf, never NaN).  MRS_ERR_UNSUPPORTED (outputs untouched) when E*N*n_rays >= 2^32 - 1.
+ * Replaces Object.raycast (Object.py:143-174). */
 int mrs_proximity(const MrsConfig* cfg, const MrsBuffers* bufs, float threshold, float* gap_agent, int* nearest,
                   float* gap_ground, unsigned char* collision, void* stream);
 int mrs_raycast(const MrsConfig* cfg, const MrsBuffers* bufs, const float* directions, int n_rays,

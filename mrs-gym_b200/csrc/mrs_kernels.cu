@@ -558,10 +558,13 @@ proximity_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, float 
         if (d2 < best) { best = d2; arg = j; }
     }
     const float ga = sqrtf(best) - 2.f * c.phys.contact_radius;
-    // ground: same support extent of the collision cylinder as the contact row of the step
+    // ground: the lowest of the four rim points (+-r, 0, cz), (0, +-r, cz), cz = -h sign(R22), that the step's ground
+    // rows use (ground_setup): r max(|R20|, |R21|) + h |R22| below the centre, plus the collision margin
     const float qx = b.state[3 * (size_t)S + s], qy = b.state[4 * (size_t)S + s];
+    const float qz = b.state[5 * (size_t)S + s], qw = b.state[6 * (size_t)S + s];
+    const float R20 = 2.f * (qx * qz - qy * qw), R21 = 2.f * (qy * qz + qx * qw);
     const float R22 = 1.f - 2.f * (qx * qx + qy * qy);
-    const float ext = c.phys.col_radius * sqrtf(fmaxf(1.f - R22 * R22, 0.f)) + c.phys.col_halfheight * fabsf(R22) +
+    const float ext = c.phys.col_radius * fmaxf(fabsf(R20), fabsf(R21)) + c.phys.col_halfheight * fabsf(R22) +
                       c.phys.col_margin;
     const float gg = z - ext - c.phys.ground_z;
     if (gap_agent) gap_agent[s] = ga;
@@ -588,6 +591,15 @@ raycast_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const fl
     float Rm[9];
     quat_to_mat(st, Rm);
     float dx = dirs[3 * r], dy = dirs[3 * r + 1], dz = dirs[3 * r + 2];
+    // only the orientation of a direction counts: it is divided by its largest component first, so that every finite
+    // nonzero magnitude (denormal to FLT_MAX) normalises like its unit vector; a zero or non-finite one hits nothing
+    const float big = fmaxf(fmaxf(fabsf(dx), fabsf(dy)), fabsf(dz));
+    if (!(big > 0.f) || !isfinite(dx) || !isfinite(dy) || !isfinite(dz)) {
+        hit_dist[tid] = INFINITY;
+        hit_id[tid] = -1;
+        return;
+    }
+    dx /= big; dy /= big; dz /= big;
     float sx = ox, sy = oy, sz = oz;
     if (body) {
         const float tx = Rm[0] * dx + Rm[1] * dy + Rm[2] * dz, ty = Rm[3] * dx + Rm[4] * dy + Rm[5] * dz,
@@ -616,7 +628,9 @@ raycast_kernel(const __grid_constant__ MrsConfig c, const MrsBuffers b, const fl
         if (j == ai) continue;
         const float cx = px[j] - sx, cy = py[j] - sy, cz = pz[j] - sz;
         const float tc = cx * dx + cy * dy + cz * dz;                  // closest approach along the ray
-        const float d2 = cx * cx + cy * cy + cz * cz - tc * tc;
+        // squared miss distance from the perpendicular itself: |c|^2 - tc^2 cancels to ~1e-3 m^2 at 100 m
+        const float ex = cx - tc * dx, ey = cy - tc * dy, ez = cz - tc * dz;
+        const float d2 = ex * ex + ey * ey + ez * ez;
         if (d2 > rad2) continue;
         const float t = tc - sqrtf(rad2 - d2);
         if (t >= 0.f && t < best) { best = t; id = j; }

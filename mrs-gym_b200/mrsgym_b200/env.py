@@ -134,7 +134,10 @@ class Environment:
         spheres come within `radius` of its own, as a bool mask [..., N, N] plus the gaps [..., N, N]."""
         sw = self.swarm
         p = sw.get_pos()
-        gap = torch.cdist(p, p) - 2.0 * float(sw.cfg.phys.contact_radius)
+        # pairwise differences, not the |a|^2 + |b|^2 - 2 a.b product form cdist takes above 25 points: that one
+        # cancels to millimetres for a swarm a few metres from the origin (and worse far from it)
+        d = torch.cdist(p, p, compute_mode='donot_use_mm_for_euclid_dist')
+        gap = d - 2.0 * float(sw.cfg.phys.contact_radius)
         eye = torch.eye(sw.N, dtype=torch.bool, device=p.device)
         mask = (gap < float(radius)) & ~eye
         return {'mask': self._out(mask), 'gap': self._out(gap)}

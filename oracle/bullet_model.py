@@ -259,6 +259,21 @@ def tournament_partner(N):
     return part
 
 
+def ground_rim(pos, R, P: PhysicsParams):
+    """The four lower-rim points of the collision cylinder (the face that looks down) for positions [E,N,3] and
+    body->world rotations [E,N,3,3]: body-frame points c [E,N,4,3], world z in the body frame nb [E,N,3] (row 2 of
+    R) and each point's gap to the ground [E,N,4] (collision margin included)."""
+    E, N = pos.shape[:2]
+    sgn = np.where(R[..., 2, 2] >= 0.0, 1.0, -1.0)
+    c = np.empty((E, N, 4, 3))                         # body-frame contact points
+    c[..., 0] = P.col_radius * RIM[:, 0]
+    c[..., 1] = P.col_radius * RIM[:, 1]
+    c[..., 2] = (-P.col_halfheight * sgn)[..., None]
+    nb = R[..., 2, :]                                  # world z in the body frame (row 2 of R)
+    zoff = np.einsum('enk,enpk->enp', nb, c)           # height of the point above the CoM
+    return c, nb, pos[..., 2, None] + zoff - P.col_margin - P.ground_z
+
+
 def solve_contacts(pos, quat, v1, w1, P: PhysicsParams, dt: float):
     """Sequential-impulse contact solve on the unconstrained velocities (see the module
     docstring for the row set and the sweep order).  Returns (v, w) world frame."""
@@ -276,14 +291,7 @@ def solve_contacts(pos, quat, v1, w1, P: PhysicsParams, dt: float):
     # ---- ground rows: four lower-rim points (the face that looks down)
     g_act = np.zeros((E, N, 4), dtype=bool)
     if P.ground_contact:
-        sgn = np.where(R[..., 2, 2] >= 0.0, 1.0, -1.0)
-        c = np.empty((E, N, 4, 3))                         # body-frame contact points
-        c[..., 0] = P.col_radius * RIM[:, 0]
-        c[..., 1] = P.col_radius * RIM[:, 1]
-        c[..., 2] = (-P.col_halfheight * sgn)[..., None]
-        nb = R[..., 2, :]                                  # world z in the body frame (row 2 of R)
-        zoff = np.einsum('enk,enpk->enp', nb, c)           # height of the point above the CoM
-        dist = pos[..., 2, None] + zoff - P.col_margin - P.ground_z
+        c, nb, dist = ground_rim(pos, R, P)
         g_act = dist < P.contact_margin
         g_bias = _contact_bias(dist, P, dt)
         g_a = np.cross(c, nb[..., None, :])                # (c x n)_body
