@@ -87,13 +87,20 @@ typedef enum {
 #define MRS_STATUS_COMM_TIMEOUT 4u /* mrs_stats_allreduce / mrs_comm_barrier gave up waiting for a peer */
 #define MRS_STATUS_NEIGHBOR_OVERFLOW 32u /* mrs_neighbors: an agent had more neighbours than max_nbr (list truncated) */
 
-/* stats slots (unsigned long long, device; summed across GPUs per rollout) */
-#define MRS_STAT_AGENT_CONTACTS 0  /* sphere-sphere contact rows that pushed         */
-#define MRS_STAT_GROUND_CONTACTS 1
-#define MRS_STAT_NONFINITE 2
-#define MRS_STAT_NAN_ACTIONS 3
-#define MRS_STAT_CONTACT_CHUNKS 4   /* N <= 32: warp-chunk steps that took the contact path (solver) */
-#define MRS_STAT_SOLVER_SWEEPS 5    /* N <= 32: Gauss-Seidel sweeps summed over those chunk steps */
+/* stats slots (unsigned long long, device; summed across GPUs per rollout; never reset by a step).  The unit of
+ * each counter is the same on every step path unless noted; a warp-chunk holds 32 / pow2ceil(N) envs. */
+#define MRS_STAT_AGENT_CONTACTS 0  /* per agent-step: sphere-sphere pair rows of the agent whose normal impulse
+                                      ended > 0 (a pushing pair counts once for each of its two agents) */
+#define MRS_STAT_GROUND_CONTACTS 1 /* agent-steps whose ground rows pushed (sum of the four normal impulses > 0) */
+#define MRS_STAT_NONFINITE 2       /* agent-steps that end with a non-finite state component */
+#define MRS_STAT_NAN_ACTIONS 3     /* agent-steps whose action has a NaN component (MRS_STATUS_NAN_ACTION) */
+#define MRS_STAT_CONTACT_CHUNKS 4  /* N <= 32 (0 otherwise): warp-chunk steps on the contact path.  Single-step
+                                      launches (mrs_step, mrs_rollout): one per chunk and step that has an agent
+                                      below the ground-skip height, a pair within contact range or a NaN action.
+                                      mrs_step_many: T - t0 per chunk whose first such step is t0 (the chunk
+                                      stays on the contact path for the rest of the launch) */
+#define MRS_STAT_SOLVER_SWEEPS 5   /* N <= 32 (0 otherwise): per contact-path chunk step, the largest number of
+                                      Gauss-Seidel sweeps among its envs */
 #define MRS_STAT_NEIGHBOR_OVERFLOW 6 /* mrs_neighbors: rows whose list was truncated at max_nbr */
 
 /* cf2x.urdf properties (mrsgym/models/cf2x.urdf:5,11-12,42-78), the derived ones of

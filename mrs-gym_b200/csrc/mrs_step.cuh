@@ -238,12 +238,15 @@ static __device__ __noinline__ void chunk_step_contact(const MrsConfig* cptr, co
         const unsigned sum_rows = __reduce_add_sync(kFull32, n_agent_rows);
         const unsigned sum_gnd = __reduce_add_sync(kFull32, n_ground);
         const unsigned max_sw = __reduce_max_sync(kFull32, n_sweeps);
+        // non-finite agents and NaN actions count per agent, like the N > 32 kernels
+        const unsigned sum_bad = __reduce_add_sync(kFull32, (status & MRS_STATUS_NONFINITE) ? 1u : 0u);
+        const unsigned sum_nan = __reduce_add_sync(kFull32, (status & MRS_STATUS_NAN_ACTION) ? 1u : 0u);
         if (lane == 0) {
             if (any_status) atomicOr(&sh_events[0], any_status);
             if (sum_rows) atomicAdd(&sh_events[1], sum_rows);
             if (sum_gnd) atomicAdd(&sh_events[2], sum_gnd);
-            if (any_status & MRS_STATUS_NONFINITE) atomicAdd(&sh_events[3], 1u);
-            if (any_status & MRS_STATUS_NAN_ACTION) atomicAdd(&sh_events[4], 1u);
+            if (sum_bad) atomicAdd(&sh_events[3], sum_bad);
+            if (sum_nan) atomicAdd(&sh_events[4], sum_nan);
             if (max_sw) atomicAdd(&sh_events[6], max_sw);
         }
     }
@@ -772,12 +775,15 @@ step_group_kernel(const __grid_constant__ MrsConfig c_in, const __grid_constant_
                 const unsigned any_status = __reduce_or_sync(kFull32, status);
                 const unsigned sum_rows = __reduce_add_sync(kFull32, n_agent_rows);
                 const unsigned sum_gnd = __reduce_add_sync(kFull32, n_ground);
+                // per agent (the status of a lane without an agent, or of a handed-off chunk, is 0 here)
+                const unsigned sum_bad = __reduce_add_sync(kFull32, (status & MRS_STATUS_NONFINITE) ? 1u : 0u);
+                const unsigned sum_nan = __reduce_add_sync(kFull32, (status & MRS_STATUS_NAN_ACTION) ? 1u : 0u);
                 if (lane == 0) {
                     if (any_status) atomicOr(&sh_events[0], any_status);
                     if (sum_rows) atomicAdd(&sh_events[1], sum_rows);
                     if (sum_gnd) atomicAdd(&sh_events[2], sum_gnd);
-                    if (any_status & MRS_STATUS_NONFINITE) atomicAdd(&sh_events[3], 1u);
-                    if (any_status & MRS_STATUS_NAN_ACTION) atomicAdd(&sh_events[4], 1u);
+                    if (sum_bad) atomicAdd(&sh_events[3], sum_bad);
+                    if (sum_nan) atomicAdd(&sh_events[4], sum_nan);
                 }
             }
         }
@@ -893,8 +899,8 @@ __device__ __forceinline__ void agent_pre(const MrsConfig& c, const Derived& d, 
 #pragma unroll
         for (int i = 0; i < 4; ++i) b.rpm[i * (size_t)S + s] = rpm[i];
     }
-    if (status && b.status) {
-        atomicOr(b.status, status);
+    if (status) {
+        if (b.status) atomicOr(b.status, status);
         if (b.stats) atomicAdd(b.stats + MRS_STAT_NAN_ACTIONS, 1ull);
     }
 }

@@ -88,6 +88,15 @@ class MrsAutoResetArgs(C.Structure):
                 ('max_rounds', C.c_int), ('episode_length', C.c_int), ('max_timesteps', C.c_int)]
 
 
+class Derived(C.Structure):
+    """mirror of the library's internal struct Derived (mrs_device.cuh), as mrs_debug_derived fills it: the constants
+    the step derives from a config (tools/gen_baked.py bakes them; the tests read thresholds from them)"""
+    _fields_ = [('inv_mass', f), ('inv_I', f * 3), ('gnd_c', f), ('dw_c', f), ('rpm2rad', f), ('q_x2', f),
+                ('cap_w2', f), ('cap_k', f), ('cap_c', f), ('lim2', f), ('gnd_skip_z', f), ('inv_dt', f),
+                ('erp_dt', f), ('s_max', f), ('comm_inf', C.c_int), ('inv_ctrl_dt', f), ('inv_4kf', f),
+                ('inv_pwm_a', f), ('inv_qmass', f)]
+
+
 class MrsError(RuntimeError):
     pass
 

@@ -274,9 +274,19 @@ def ground_rim(pos, R, P: PhysicsParams):
     return c, nb, pos[..., 2, None] + zoff - P.col_margin - P.ground_z
 
 
-def solve_contacts(pos, quat, v1, w1, P: PhysicsParams, dt: float):
+def solve_contacts(pos, quat, v1, w1, P: PhysicsParams, dt: float, counts: dict | None = None):
     """Sequential-impulse contact solve on the unconstrained velocities (see the module
-    docstring for the row set and the sweep order).  Returns (v, w) world frame."""
+    docstring for the row set and the sweep order).  Returns (v, w) world frame.
+
+    counts (optional dict): filled with what the kernels count (include/mrs_b200.h, stats slots), shaped like the
+    leading dims of pos:
+      'sweeps'    [...]     sweeps run while the env was alive (0 for an env that had no row when no env had one);
+      'active'    [...]     the env had an active row (ground point within the margin, or a pair in range);
+      'worst'     [s][...]  largest row change of every sweep s (all envs, alive or not);
+      'ground'    [..., N]  the agent's ground rows pushed (sum of its four normal impulses > 0);
+      'pair_rows' [..., N]  pair rows of the agent with normal impulse > 0 (a pushing pair counts for both agents);
+      'g_lam'     [..., N, 4] final normal impulses of the ground rows (0 where no row);
+      'p_lam'     list of [...] final normal impulses of the active pair rows (inactive rows are 0)."""
     lead = pos.shape[:-2]
     N = pos.shape[-2]
     pos = pos.reshape(-1, N, 3)
@@ -316,10 +326,19 @@ def solve_contacts(pos, quat, v1, w1, P: PhysicsParams, dt: float):
         rounds.append(dict(lo=lo, hi=hi, act=act, n=n, t1=t1, t2=t2,
                            bias=_contact_bias(dd - 2.0 * P.contact_radius, P, dt),
                            lam=np.zeros(act.shape), lt1=np.zeros(act.shape), lt2=np.zeros(act.shape)))
+    if counts is not None:
+        p_act = np.zeros(E, dtype=bool)
+        for rd in rounds:
+            p_act |= rd['act'].any(axis=-1)
+        counts.update(sweeps=np.zeros(lead, np.int64), active=(g_act.any(axis=(-2, -1)) | p_act).reshape(lead),
+                      worst=[], ground=np.zeros(lead + (N,), bool), pair_rows=np.zeros(lead + (N,), np.int64),
+                      g_lam=np.zeros(lead + (N, 4)), p_lam=[])
     if not (g_act.any() or rounds):
         return np.array(v1, np.float64).reshape(lead + (N, 3)), np.array(w1, np.float64).reshape(lead + (N, 3))
     alive = np.ones(E, dtype=bool)                         # envs that have not converged yet
+    sweeps = np.zeros(E, np.int64)
     for it in range(int(P.solver_iters)):
+        sweeps += alive
         worst = np.zeros(E)
         am = alive[:, None]
         if P.ground_contact:
@@ -355,9 +374,23 @@ def solve_contacts(pos, quat, v1, w1, P: PhysicsParams, dt: float):
                 v[:, hi] -= u * (dl * im)[..., None]
                 if dl.shape[1]:
                     worst = np.maximum(worst, np.max(np.abs(dl) * 2.0 * im, axis=-1))
+        if counts is not None:
+            counts['worst'].append(worst.reshape(lead))
         alive = alive & ~(worst < P.solver_tol)
         if not alive.any():
             break
+    if counts is not None:
+        counts['sweeps'] = sweeps.reshape(lead)
+        pair_rows = np.zeros((E, N), np.int64)
+        for rd in rounds:
+            pushed = (rd['lam'] > 0.0).astype(np.int64)
+            pair_rows[:, rd['lo']] += pushed
+            pair_rows[:, rd['hi']] += pushed
+            counts['p_lam'].append(np.where(rd['act'], rd['lam'], 0.0).reshape(lead + (-1,)))
+        counts['pair_rows'] = pair_rows.reshape(lead + (N,))
+        if P.ground_contact:
+            counts['ground'] = (np.sum(g_lam, axis=-1) > 0.0).reshape(lead + (N,))
+            counts['g_lam'] = g_lam.reshape(lead + (N, 4))
     w = matvec(R, wb)
     return v.reshape(lead + (N, 3)), w.reshape(lead + (N, 3))
 
@@ -380,11 +413,12 @@ def integrate_positions(pos, quat, v, w, P: PhysicsParams, dt: float):
 
 
 def bullet_step(pos, quat, vel, angvel, force_w, torque_w, P: PhysicsParams,
-                dt: float = 0.01, gravity: float = 9.81):
+                dt: float = 0.01, gravity: float = 9.81, counts: dict | None = None):
     """One ``stepSimulation`` (numSubSteps=0).  Inputs float64, world frame; force/torque
-    are the summed external wrench about the CoM.  Returns (pos, quat, vel, angvel)."""
+    are the summed external wrench about the CoM.  Returns (pos, quat, vel, angvel).
+    counts: see solve_contacts (left empty when both contact kinds are off)."""
     v1, w1 = unconstrained_velocities(quat, vel, angvel, force_w, torque_w, P, dt, gravity)
     if P.ground_contact or P.agent_contact:
-        v1, w1 = solve_contacts(pos, quat, v1, w1, P, dt)
+        v1, w1 = solve_contacts(pos, quat, v1, w1, P, dt, counts)
     pos1, q1 = integrate_positions(pos, quat, v1, w1, P, dt)
     return pos1, q1, v1, w1

@@ -181,6 +181,13 @@ class SpecEnv:
         if 'last_vel_e' not in c:
             c['last_vel_e'] = vel_e
             c['d_vel_e'] = np.zeros((self.E, self.N, 3))
+        elif np.isnan(c['last_vel_e'][..., 0]).any():
+            # rows of agents whose controller has never run (step(nan_policy='agent_none') put the marker back):
+            # their first call, per agent, like the device's last_vel_e.x = NaN marker
+            first = np.isnan(c['last_vel_e'][..., 0])[..., None]
+            c['last_vel_e'] = np.where(first, vel_e, c['last_vel_e'])
+            c['d_vel_e'] = np.where(first, 0.0, c['d_vel_e'])
+            c['last_target_vel'] = np.where(first, target_vel, c['last_target_vel'])
         if 'last_target_vel' not in c:
             c['last_target_vel'] = target_vel
         if 'integral_vel_e' not in c:
@@ -265,13 +272,23 @@ class SpecEnv:
         return forces.astype(np.float64), z_torque.astype(np.float64)
 
     # ---- one env.step (MRS.step, /root/reference/mrsgym/MRS.py:240-277)
-    def step(self, actions, action_type=None):
+    def step(self, actions, action_type=None, nan_policy='raise', counts=None):
+        """nan_policy: 'raise' (MRS.py:247-248) or 'agent_none', the rule of the CUDA step for device-resident actions:
+        an agent with a NaN in any action component steps like MRS.step(None) -- no rotor wrench (thrust, drag,
+        ground effect) and no downwash received, its controller state as before the step, its rotor speeds 0 -- while
+        it still casts downwash onto the others.  counts: see bullet_model.solve_contacts."""
         mode = action_type or self.action_type
         Q, E, N = self.Q, self.E, self.N
+        nan_rows = None
         if actions is not None:
             actions = np.asarray(actions)
             if np.any(np.isnan(actions)):
-                raise Exception('The given action contains NaN')
+                if nan_policy != 'agent_none':
+                    raise Exception('The given action contains NaN')
+                actions = actions.reshape(E, N, -1)
+                nan_rows = np.any(np.isnan(actions), axis=-1)
+                actions = np.where(nan_rows[..., None], actions.dtype.type(0), actions)
+                saved = {k: np.array(v, copy=True) for k, v in self.ctrl.items()}
             actions = actions.reshape(E, N, -1)
             if mode == 'set_target_vel':
                 rpm = self._vel_control(actions)
@@ -291,12 +308,27 @@ class SpecEnv:
                 raise AttributeError("'Quadcopter' object has no attribute '%s'" % mode)
             forces, z_torque = self._apply_speeds(rpm)
             Fw, Tw = self._wrench(forces, z_torque)
+            if nan_rows is not None:
+                Fw[nan_rows] = 0.0
+                Tw[nan_rows] = 0.0
+                self.speeds = np.array(self.speeds, np.float64)
+                self.speeds[nan_rows] = 0.0
+                for k in list(self.ctrl):
+                    v = np.array(np.broadcast_to(self.ctrl[k], (E, N, 3)), copy=True)
+                    if k in saved:
+                        v[nan_rows] = saved[k][nan_rows]
+                    elif nan_rows.all():
+                        del self.ctrl[k]
+                        continue
+                    else:       # created by this step: the agents back to "never called"
+                        v[nan_rows] = np.nan if k == 'last_vel_e' else 0.0
+                    self.ctrl[k] = v
         else:
             Fw = np.zeros((E, N, 3))
             Tw = np.zeros((E, N, 3))
         self.last = dict(rpm=np.array(self.speeds, np.float64), force=Fw, torque=Tw)
         self.pos, self.quat, self.vel, self.angvel = bm.bullet_step(
-            self.pos, self.quat, self.vel, self.angvel, Fw, Tw, self.P, self.dt, self.gravity)
+            self.pos, self.quat, self.vel, self.angvel, Fw, Tw, self.P, self.dt, self.gravity, counts)
         X = self.calc_X()
         self.X.insert(0, X)
         del self.X[self.K + 1:]
