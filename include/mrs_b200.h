@@ -32,6 +32,25 @@
  *                         also the per-slice partial sums of the pair pass).  P =
  *                         mrs_scratch_planes(E, N): 7, or 7 + 2 * slices (<= 32 slices; 1 when
  *                         E is large) for N > 128.  No initial contents required.
+ *   wrench float[6][S]    optional (may be NULL) external wrench per agent, SoA planes like state: force fx fy fz
+ *                         [N] at the centre of mass (planes 0-2), torque tx ty tz [N m] (planes 3-5), both in the
+ *                         WORLD frame.  It enters the Bullet step where the rotor / aero wrench does, in the
+ *                         unconstrained velocities before the contact solve:
+ *                           v* = clamp(v + dt ((R Fb + F_ext) / m - g z - damping), +-max_coord_vel)
+ *                           w*: the body-frame right-hand side gains R^T tau_ext before I^-1
+ *                         so it takes part in the contact solve like any other applied force (a grounded agent
+ *                         pressed down stays put, a sideways push meets friction).  The buffer persists: every step
+ *                         of every stepping call (mrs_step, each of the T steps of mrs_step_many / mrs_rollout /
+ *                         mrs_rollout_host, mrs_step_host) reads it until the caller changes it -- unlike
+ *                         p.applyExternalForce, which Bullet clears after each stepSimulation.  mrs_set_state,
+ *                         mrs_spawn and mrs_autoreset leave it alone.  An agent with a NaN action loses its rotor
+ *                         wrench and the downwash it receives but keeps the external wrench.  A NaN / inf component
+ *                         is not special-cased: like any non-finite acceleration it meets the +-max_coord_vel clamp
+ *                         (fminf / fmaxf return the bound for NaN), so that agent moves at the clamp velocity and
+ *                         stays finite (no MRS_STATUS_NONFINITE); no other agent is affected.  NULL: no
+ *                         external wrench, the step runs exactly the kernels it runs without this member.  With a
+ *                         wrench, N <= 32 runs the run-time-width kernel on small CTAs (no baked constants, no
+ *                         chained hand-over in mrs_rollout).
  */
 #ifndef MRS_B200_H
 #define MRS_B200_H
@@ -42,7 +61,7 @@
 extern "C" {
 #endif
 
-#define MRS_ABI_VERSION 5
+#define MRS_ABI_VERSION 6
 #define MRS_STATE_PLANES 13
 #define MRS_CTRL_PLANES 18
 #define MRS_STATS_SLOTS 8
@@ -164,6 +183,7 @@ typedef struct {
     unsigned long long* stats;           /* [MRS_STATS_SLOTS] */
     unsigned long long* sync;            /* [MRS_SYNC_WORDS], zero-initialised once by the caller, owned by the library
                                             afterwards; NULL = mrs_rollout falls back to grid-wide dependencies */
+    float* wrench;                       /* [6][S] or NULL: external force / torque per agent, world frame (see above) */
 } MrsBuffers;
 
 int mrs_abi_version(void);
@@ -202,14 +222,14 @@ int mrs_debug_derived(const MrsConfig* cfg, void* out, size_t out_bytes);
  * effect, drag, downwash) -> Bullet step (contact) -> newest X slice into X tape slot
  * `slot_x`, newest A slice into A tape slot `slot_a` (the reference shifts its X and A deques
  * independently, MRS.py:87-114).  actions: device float[E][N][ACTION_DIM] (ignored for
- * MRS_NO_ACTION).
+ * MRS_NO_ACTION).  bufs->wrench (NULL or [6][S]) is added to every agent's wrench in this step.
  * Replaces MRS.step's set_actions + step_sim + calc_Xk + calc_Ak (MRS.py:252-257). */
 int mrs_step(const MrsConfig* cfg, const MrsBuffers* bufs, const float* actions, int slot_x, int slot_a,
              void* stream);
 
 /* T consecutive steps in one call (N <= 32: one launch, state stays in registers); step t
  * reads actions[t] (device float[T][E][N][ACTION_DIM]) and writes tape slots
- * slot_x_first - t / slot_a_first - t.  The rollout loop of
+ * slot_x_first - t / slot_a_first - t.  Every step reads the same bufs->wrench.  The rollout loop of
  * examples/simulating_data/helper/DataGenerator.py:8-48 with pre-computed actions. */
 int mrs_step_many(const MrsConfig* cfg, const MrsBuffers* bufs, const float* actions, int T,
                   int slot_x_first, int slot_a_first, void* stream);
@@ -219,7 +239,8 @@ int mrs_step_many(const MrsConfig* cfg, const MrsBuffers* bufs, const float* act
  * mrs_step_many.  For N in {8, 16, 32} and jobs that fill the GPU the launches are CHAINED: environments are
  * independent, so the chunk range a CTA of step t has finished is handed to a CTA of step t+1 through
  * bufs->sync (a queue in completion order) instead of waiting for the whole grid of step t -- an SM never waits
- * for the slowest SM of the previous step.  Everything else behaves like T calls of mrs_step.  Capturable in a
+ * for the slowest SM of the previous step (not with bufs->wrench set: then every step is a plain launch of the
+ * wrench kernel).  Everything else behaves like T calls of mrs_step, the wrench included.  Capturable in a
  * CUDA graph.  The rollout loop of examples/simulating_data/helper/DataGenerator.py:8-48. */
 int mrs_rollout(const MrsConfig* cfg, const MrsBuffers* bufs, const float* actions, int T, int slot_x_first,
                 int slot_a_first, void* stream);
@@ -264,8 +285,8 @@ int mrs_tape_fill(const MrsConfig* cfg, const MrsBuffers* bufs, int which, int s
 /* End-to-end step over HOST buffers (pinned recommended): H2D actions, mrs_step, D2H of the
  * newest X slice ([E][N][D]) and A slice ([E][N][N], and / or its bit-packed form, see mrs_pack_adjacency); X_host /
  * A_host / Abits_host may be NULL.
- * dev_actions: caller-owned device staging float[E][N][ACTION_DIM].  Synchronises the
- * stream before returning (the reference's step is synchronous). */
+ * dev_actions: caller-owned device staging float[E][N][ACTION_DIM].  bufs->wrench applies as in mrs_step (it stays
+ * on the device; no copy).  Synchronises the stream before returning (the reference's step is synchronous). */
 int mrs_step_host(const MrsConfig* cfg, const MrsBuffers* bufs, const float* actions_host,
                   float* dev_actions, float* X_host, float* A_host, unsigned int* Abits_host,
                   unsigned int* dev_Abits, int slot_x, int slot_a, void* stream);
@@ -357,8 +378,8 @@ int mrs_raycast(const MrsConfig* cfg, const MrsBuffers* bufs, const float* direc
  * float[T][E][N][ACTION_DIM] (pinned), dev_actions: caller-owned device staging, TWO action
  * buffers float[2][E][N][ACTION_DIM]; X_host float[T][E][N][D] / A_host float[T][E][N][N] (pinned,
  * may be NULL) receive the newest slice of every step.  Step t writes tape slots
- * slot_x_first - t / slot_a_first - t (the caller guarantees they exist).  Synchronises before
- * returning.  The open-loop rollout of examples/simulating_data/helper/DataGenerator.py:8-48 for a
+ * slot_x_first - t / slot_a_first - t (the caller guarantees they exist); every step reads bufs->wrench.
+ * Synchronises before returning.  The open-loop rollout of examples/simulating_data/helper/DataGenerator.py:8-48 for a
  * caller whose actions and trajectory buffers live in host memory. */
 int mrs_rollout_host(const MrsConfig* cfg, const MrsBuffers* bufs, const float* actions_host,
                      float* dev_actions, float* X_host, float* A_host, unsigned int* Abits_host,

@@ -34,6 +34,18 @@ struct StepArgs {
 };
 
 // ------------------------------------------------------------------------------ state planes
+// the six external wrench components of agent slot s (MrsBuffers.wrench, [6][S]): read-only for the whole launch
+__device__ __forceinline__ ExtWrench load_wrench(const float* __restrict__ w, unsigned S, unsigned s) {
+    ExtWrench x;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        x.f[k] = __ldg(w + (size_t)k * S + s);
+        x.t[k] = __ldg(w + (size_t)(3 + k) * S + s);
+    }
+    return x;
+}
+
+
 __device__ __forceinline__ void load_agent(const float* __restrict__ st, unsigned S, unsigned s, Agent& a) {
     a.px = st[0 * S + s]; a.py = st[1 * S + s]; a.pz = st[2 * S + s];
     a.qx = st[3 * S + s]; a.qy = st[4 * S + s]; a.qz = st[5 * S + s]; a.qw = st[6 * S + s];

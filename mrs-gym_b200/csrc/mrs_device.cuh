@@ -296,12 +296,20 @@ __device__ __forceinline__ float downwash_pair(const MrsQuadParams& q, const Der
     return (rz > 0.f && dxy2 < 100.f) ? f : 0.f;
 }
 
+// The caller's external wrench of one agent (MrsBuffers.wrench): force at the CoM and torque, both world frame.
+struct ExtWrench {
+    float f[3], t[3];
+};
+
 // rotor thrust + yaw torque (Quadcopter.py:38-45), ground effect / drag (Quadcopter.py:69-98),
 // downwash sum `dw` -> Bullet unconstrained velocity update (bullet_model.unconstrained_velocities).
+// EXT: the external wrench xw joins the applied wrench (force after the rotation of the body-frame sum, torque
+// rotated into the body frame before I^-1), so the contact solve sees it like any other applied force.  Without
+// EXT the code is the one of the kernels that never read a wrench (x + 0 does not fold under IEEE rules).
 // Overwrites s.v / s.w with the unconstrained velocities v*, w*.
-template <bool FORCES>
+template <bool FORCES, bool EXT = false>
 __device__ __forceinline__ void apply_wrench(const MrsConfig& c, const Derived& d, Agent& s, const float* R,
-                                             const float* rpm, float dw) {
+                                             const float* rpm, float dw, const ExtWrench& xw = ExtWrench{}) {
     const MrsQuadParams& q = c.quad;
     const MrsPhysicsParams& ph = c.phys;
     float Fb[3] = {0.f, 0.f, 0.f}, Tb[3] = {0.f, 0.f, 0.f};
@@ -328,13 +336,25 @@ __device__ __forceinline__ void apply_wrench(const MrsConfig& c, const Derived& 
         Fb[1] = R[3] * cx + R[4] * cy + R[5] * cz;
         Fb[2] = R[6] * cx + R[7] * cy + R[8] * cz + fz + dw;
     }
-    // linear: a = R Fb / m - g z - v (k + k|v|)
+    if constexpr (EXT) {    // external torque, world -> body: R^T tau
+        Tb[0] += R[0] * xw.t[0] + R[3] * xw.t[1] + R[6] * xw.t[2];
+        Tb[1] += R[1] * xw.t[0] + R[4] * xw.t[1] + R[7] * xw.t[2];
+        Tb[2] += R[2] * xw.t[0] + R[5] * xw.t[1] + R[8] * xw.t[2];
+    }
+    // linear: a = (R Fb + F_ext) / m - g z - v (k + k|v|)
     const float im = d.inv_mass;
     const float vn = fast_sqrt(s.vx * s.vx + s.vy * s.vy + s.vz * s.vz);
     const float kl = ph.lin_damping + ph.lin_damping * vn;
-    const float ax = (R[0] * Fb[0] + R[1] * Fb[1] + R[2] * Fb[2]) * im - s.vx * kl;
-    const float ay = (R[3] * Fb[0] + R[4] * Fb[1] + R[5] * Fb[2]) * im - s.vy * kl;
-    const float az = (R[6] * Fb[0] + R[7] * Fb[1] + R[8] * Fb[2]) * im - c.gravity - s.vz * kl;
+    float ax, ay, az;
+    if constexpr (EXT) {
+        ax = ((R[0] * Fb[0] + R[1] * Fb[1] + R[2] * Fb[2]) + xw.f[0]) * im - s.vx * kl;
+        ay = ((R[3] * Fb[0] + R[4] * Fb[1] + R[5] * Fb[2]) + xw.f[1]) * im - s.vy * kl;
+        az = ((R[6] * Fb[0] + R[7] * Fb[1] + R[8] * Fb[2]) + xw.f[2]) * im - c.gravity - s.vz * kl;
+    } else {
+        ax = (R[0] * Fb[0] + R[1] * Fb[1] + R[2] * Fb[2]) * im - s.vx * kl;
+        ay = (R[3] * Fb[0] + R[4] * Fb[1] + R[5] * Fb[2]) * im - s.vy * kl;
+        az = (R[6] * Fb[0] + R[7] * Fb[1] + R[8] * Fb[2]) * im - c.gravity - s.vz * kl;
+    }
     // angular in the body frame: I wdot = tau - w x Iw - Iw (k + k|w|)
     const float wb[3] = {R[0] * s.wx + R[3] * s.wy + R[6] * s.wz, R[1] * s.wx + R[4] * s.wy + R[7] * s.wz,
                          R[2] * s.wx + R[5] * s.wy + R[8] * s.wz};

@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('MRS_B200_LIB') or os.path.join(_HERE, 'libmrs_b200.so')   # override: A/B builds
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 STATE_PLANES = 13
 CTRL_PLANES = 18
 STATS_SLOTS = 8
@@ -79,7 +79,7 @@ class MrsConfig(C.Structure):
 class MrsBuffers(C.Structure):
     _fields_ = [('state', C.c_void_p), ('ctrl', C.c_void_p), ('rpm', C.c_void_p),
                 ('X_tape', C.c_void_p), ('A_tape', C.c_void_p), ('scratch', C.c_void_p),
-                ('status', C.c_void_p), ('stats', C.c_void_p), ('sync', C.c_void_p)]
+                ('status', C.c_void_p), ('stats', C.c_void_p), ('sync', C.c_void_p), ('wrench', C.c_void_p)]
 
 
 class MrsAutoResetArgs(C.Structure):

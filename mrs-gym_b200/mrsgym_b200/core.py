@@ -86,6 +86,8 @@ class Swarm:
     nbr = None
     N_idx = None
     N_cnt = None
+    # external force / torque per agent, float32 [6, S] (set_external_wrench); the step reads it while it is bound
+    wrench = None
 
     def __init__(self, E: int, N: int, K: int = 0, action_type='set_target_vel', state_layout=_abi.X_POS_VEL,
                  comm_range=float('inf'), dt=0.01, gravity=9.81, agent_radius=0.3, device='cuda', contact_radius=None,
@@ -179,6 +181,7 @@ class Swarm:
         b.scratch = self.scratch.data_ptr() if self.scratch is not None else None
         b.status, b.stats = self.status.data_ptr(), self.stats.data_ptr()
         b.sync = self.sync.data_ptr()
+        b.wrench = None             # bound by set_external_wrench
 
     def _stream(self):
         if torch.cuda.current_device() != self.device.index:
@@ -546,6 +549,38 @@ class Swarm:
                 self.a_empty = False
             done += n
 
+    # ------------------------------------------------------------------ external wrench
+    def set_external_wrench(self, force=None, torque=None, env_mask=None):
+        """External force [N] at the centre of mass and torque [N m] per agent, both in the world frame
+        (MrsBuffers.wrench): PyBullet's applyExternalForce(body, -1, F, com, WORLD_FRAME) + applyExternalTorque(body,
+        -1, tau, WORLD_FRAME).  Unlike PyBullet, the wrench persists: every following step of every stepping call
+        applies it until it is changed or cleared; set_state, spawn, autoreset and MRS.reset leave it alone.
+        force / torque broadcast to [E, N, 3] ([3]: the same for every agent, [E, 1, 3]: per env); None keeps that
+        half as it is.  env_mask (bool / uint8 [E]): write only the selected envs.  The first call allocates the
+        [6, S] buffer (zeros) and binds it; later calls are in-place device copies with no allocation of the buffer
+        and no host synchronisation, so a policy may call this inside rollout(graph=True)."""
+        if self.wrench is None:
+            self.wrench = torch.zeros(6, self.S, device=self.device, dtype=torch.float32)
+        mask = None
+        if env_mask is not None:
+            mask = torch.as_tensor(env_mask, device=self.device).to(torch.bool).reshape(1, self.E, 1)
+        for lo, x in ((0, force), (3, torque)):
+            if x is None:
+                continue
+            src = torch.as_tensor(x, dtype=torch.float32, device=self.device).expand(self.E, self.N, 3).permute(2, 0, 1)
+            dst = self.wrench[lo:lo + 3].view(3, self.E, self.N)
+            dst.copy_(src if mask is None else torch.where(mask, src, dst))
+        self.bufs.wrench = self.wrench.data_ptr()
+
+    def clear_external_wrench(self):
+        """Unbind the external wrench: the step runs the kernels without one again.  The buffer is kept (a later
+        set_external_wrench writes into the same memory), so its address stays fixed."""
+        self.bufs.wrench = None
+
+    @property
+    def wrench_bound(self):
+        return bool(self.bufs.wrench)
+
     # ------------------------------------------------------------------ state access
     def set_state(self, pos=None, ori=None, vel=None, angvel=None, env_mask=None):
         """Environment.set_state -> Object.set_state (Environment.py:97-103, Object.py:42-65).
@@ -761,6 +796,7 @@ class GraphRollout:
         if actions is not None and tuple(actions.shape[:3]) != (T, sw.E, sw.N):
             raise ValueError('actions must be [T, E, N, A]')
         self.T, self.actions = T, actions
+        self.wrench = sw.bufs.wrench        # the captured kernels read the wrench iff it was bound at capture
         sw.ring = True
         self.launches_per_replay = 0
         torch.cuda.synchronize(sw.device)
@@ -771,7 +807,7 @@ class GraphRollout:
             # warm-up outside capture (lazy module load, per-function attributes): it advances the swarm by T
             # steps, so everything a later step can read is put back afterwards -- state, PID planes, counters
             # and the K+1 observation windows (the rest of the tapes is history nobody can reach any more)
-            keep = [(t, t.clone()) for t in (sw.state, sw.ctrl, sw.status, sw.stats, sw.rpm) if t is not None]
+            keep = [(t, t.clone()) for t in (sw.state, sw.ctrl, sw.status, sw.stats, sw.rpm, sw.wrench) if t is not None]
             for tape, which in ((sw.X_tape, 1), (sw.A_tape, 2), (sw.N_idx, 2), (sw.N_cnt, 2)):
                 if tape is not None:
                     keep += [(tape[sl], tape[sl].clone()) for sl in sw.window_slots(which)]
@@ -800,6 +836,9 @@ class GraphRollout:
             sw.allreduce_stats(self.stats_comm)
 
     def replay(self):
+        if self.swarm.bufs.wrench != self.wrench:
+            raise RuntimeError('the external wrench was %s since this rollout was captured: its kernels %s; capture '
+                               'again' % (('bound', 'ignore it') if self.swarm.bufs.wrench else ('unbound', 'would read it')))
         self.graph.replay()
         self.swarm.launches += self.launches_per_replay
         self.swarm.a_empty = False

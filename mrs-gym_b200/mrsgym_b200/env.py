@@ -518,6 +518,18 @@ class MRS:
         self.last_obs = Xk
         return Xk
 
+    def set_external_wrench(self, force=None, torque=None, env_mask=None):
+        """External force [N] at the centre of mass and torque [N m] per agent, world frame: wind, a push, a payload
+        (PyBullet: applyExternalForce(body, -1, F, com, WORLD_FRAME) + applyExternalTorque(body, -1, tau,
+        WORLD_FRAME)).  Shapes broadcast to [N_ENVS, N_AGENTS, 3] ([N, 3] per agent when unbatched, [3] uniform);
+        None keeps that half.  It persists across steps and reset() until changed or cleared (PyBullet clears it after
+        every stepSimulation: write it before every step to emulate that).  See Swarm.set_external_wrench."""
+        self.swarm.set_external_wrench(force, torque, env_mask)
+
+    def clear_external_wrench(self):
+        """Back to no external wrench (the step runs its kernels without one)."""
+        self.swarm.clear_external_wrench()
+
     def reset(self, pos=None, ori=None, vel=None, angvel=None, env_mask=None):
         """MRS.reset (MRS.py:174-192).  PID integrators are NOT reset (reference behaviour).
         env_mask ([E] bool) resets only the selected envs of the batch and keeps the rings of the rest.

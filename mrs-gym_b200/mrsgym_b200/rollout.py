@@ -156,7 +156,8 @@ def closed_loop_graph(env, policy, T, episode_length=None, record=('X', 'A', 'ac
     sp = env.START_POS
     spawn = (env.SEED, env._env_offset(), getattr(sp, 'z_low', None), getattr(sp, 'z_high', None),
              getattr(sp, 'xy_radius', None))
-    key = (policy, int(T), episode_length, tuple(record), sw.hx, sw.ha, env._cfg_key, env.ACTION_TYPE, spawn)
+    # the captured step kernels read the external wrench iff it was bound at capture
+    key = (policy, int(T), episode_length, tuple(record), sw.hx, sw.ha, env._cfg_key, env.ACTION_TYPE, spawn, sw.bufs.wrench)
     g = env._graphs.get(key)
     if g is None:
         g = env._graphs[key] = ClosedLoopGraph(env, policy, T, episode_length, record)
@@ -303,8 +304,9 @@ class ClosedLoopGraph:
         side = torch.cuda.Stream(device=sw.device)
         side.wait_stream(torch.cuda.current_stream(sw.device))
         with torch.cuda.stream(side):
-            keep = [(t, t.clone()) for t in (sw.state, sw.ctrl, sw.status, sw.stats, sw.rpm, env.episode, self.steps,
-                                             self.failed) if t is not None]
+            keep = [(t, t.clone()) for t in (sw.state, sw.ctrl, sw.status, sw.stats, sw.rpm, sw.wrench, env.episode,
+                                             self.steps, self.failed) if t is not None]
+            bound = sw.bufs.wrench
             for tape, which in ((sw.X_tape, 1), (sw.A_tape, 2)):
                 if tape is not None:
                     keep += [(tape[sl], tape[sl].clone()) for sl in sw.window_slots(which)]
@@ -314,6 +316,9 @@ class ClosedLoopGraph:
             for dst, src in keep:
                 dst.copy_(src)
             sw.hx, sw.ha, sw.a_empty, sw.launches, env.last_obs, env.last_action = host
+            if sw.bufs.wrench != bound:
+                raise RuntimeError('the policy bound or cleared the external wrench: bind it (set_external_wrench) '
+                                   'before rollout(graph=True); inside the loop only write it')
             torch.cuda.synchronize(sw.device)
             # an MRS is a reference cycle (its default done_fn is one of its bound methods), so a dropped env and the
             # CUDA graphs it cached are freed by the cyclic collector; freeing a graph or its memory pool while this
